@@ -23,6 +23,11 @@ cpu_baseline / --impl reference: the UNMODIFIED reference (`oracle/_ref/ziggy`, 
           same configuration, each step a bounded sample (8 of the step's 64 right-hand sides); falls back to the CPU
           oracle port (oracle/ziggy_oracle.py) when the staged reference is absent.
 
+--dump-outputs DIR: after the timed steps, the solution the last timed step returned (B x M, fp32) is written as
+          DIR/pcg_x_sample.npy at a fixed seeded sample of its grid points (all right-hand sides, DUMP_POINTS columns);
+          the inputs are seeded, so two builds run with the same arguments can be compared output for output.  With
+          N > 1 only rank 0 writes, so the file holds rank 0's right-hand sides (generator seed 42).
+
 N > 1 (torchrun): right-hand sides are independent, so each rank solves its own B = 64 shard with no data-path
 collective ("weak" scaling); time = max over ranks.  The two paths that DO need collectives are measured in the same run
 and reported as extra keys: `svi_cfg3` (observation-sharded mean-field natural-gradient step, one packed all-reduce per
@@ -48,6 +53,7 @@ E2E_GROUP = int(os.environ.get("HIPGP_E2E_GROUP", "8"))     # right-hand sides i
 CPU_SAMPLE_B = 8       # right-hand sides per CPU step: ~7 s per step on 16 cores, so that --steps 20 --warmup 5 ends in ~3 minutes
 N_MATVEC = 2 * MAXITER + 1
 METRIC = "toeplitz_matvec_GBps_in_pcg_1e6grid"
+DUMP_POINTS = 1 << 17  # grid points kept by --dump-outputs: 64 x 131072 fp32 = 32 MB
 
 
 def workload_config():
@@ -77,6 +83,17 @@ def first_row(dtype, device):
     g1 = torch.linspace(0, 4, GRID[0], dtype=dtype, device=device)
     g2 = torch.linspace(-2, 2, GRID[1], dtype=dtype, device=device)
     return hk.first_row([g1, g2], hk.Matern(nu=2.5, dtype=dtype), (SIG2, ELL), jitter=JITTER)
+
+
+def dump_outputs(path, x):
+    """Writes the solution x (B, M) at the grid points np.random.default_rng(0).choice(M, DUMP_POINTS, replace=False),
+    sorted, as path/pcg_x_sample.npy (B, DUMP_POINTS) in x's dtype."""
+    import numpy as np
+    import torch
+    cols = np.sort(np.random.default_rng(0).choice(x.shape[1], min(DUMP_POINTS, x.shape[1]), replace=False))
+    sample = x[:, torch.from_numpy(cols).to(x.device)].cpu().numpy()
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "pcg_x_sample.npy"), sample)
 
 
 class ClockSampler(threading.Thread):
@@ -503,6 +520,11 @@ def run_gpu(args):
     def step_dev():
         return plan.pcg(b, maxiter=MAXITER, tol=TOL, precond=True)
 
+    last = [None]
+
+    def step_dev_kept():          # --dump-outputs: the timed steps keep what they return
+        last[0] = step_dev()
+
     def step_e2e():
         return plan.pcg_host(b_host, x_host, maxiter=MAXITER, tol=TOL, precond=True, group=E2E_GROUP)
 
@@ -527,9 +549,10 @@ def run_gpu(args):
         step_dev()
     m0 = sampler.mark() if sampler else 0
     l0 = plan.launch_count()
-    ms_total = timed(step_dev, args.steps)
+    ms_total = timed(step_dev_kept if args.dump_outputs else step_dev, args.steps)
     launches = plan.launch_count() - l0
     m1 = sampler.mark() if sampler else 0
+    x_timed, last[0] = last[0], None      # what the last timed step returned (None without --dump-outputs)
 
     # e2e (headline): a stream of `steps` batches through the asynchronous host entry points, two in flight -- every step's
     # right-hand sides are uploaded from pinned memory and its solution downloaded inside the timed region; the upload of step
@@ -574,6 +597,9 @@ def run_gpu(args):
     plan.profile(False)
     m2 = sampler.mark() if sampler else 0
     clocks = sampler.finish(m0, m1, m0, m2) if sampler else None
+    if x_timed is not None and rank == 0:
+        dump_outputs(args.dump_outputs, x_timed)
+    del x_timed
 
     # companions (not the headline; same step definition): one right-hand side, plain matvecs, fp64, cuFFT comparison point
     extra = {}
@@ -754,7 +780,12 @@ def main():
     ap.add_argument("--other-configs", action="store_true", help="with --impl reference: time the other BASELINE configurations instead")
     ap.add_argument("--section-timeout", type=int, default=420, help="watchdog for the multi-GPU sections (seconds)")
     ap.add_argument("--cpu-sample-b", type=int, default=CPU_SAMPLE_B, help="right-hand sides per CPU step (bounded sample)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the last timed step's solution to DIR/*.npy (rank 0's right-hand sides)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; it does not apply to --impl reference")
     if args.impl == "reference":
         if args.other_configs:
             run_reference_other(args)

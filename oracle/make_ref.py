@@ -1,10 +1,12 @@
 """Stage the UNMODIFIED reference package into the git-ignored `oracle/_ref/` so that it travels to the GPU box.
 TEST / BASELINE INFRASTRUCTURE ONLY -- nothing under `hipgp_b200/` may import it.
 
-    python oracle/make_ref.py            # copies /root/reference/ziggy and run_solve_kn_experiment.py, byte for byte
+    python oracle/make_ref.py            # copies <root>/ziggy and run_solve_kn_experiment.py, byte for byte
 
-`/root/reference` exists only in the build container.  The GPU box receives the repository snapshot, which includes
-git-ignored paths (like the built `.so`), so `oracle/_ref/ziggy` is what
+<root> is the reference checkout: $HIPGP_REFERENCE_ROOT when set, else the `reference_path` that BASELINE.json records.
+
+The reference is not part of this repository.  A copy of the working tree that includes git-ignored paths (like the
+built `.so`) carries the staged copy along, so `oracle/_ref/ziggy` is what
 
   * `tests/test_gpu_dropin.py` imports after `hipgp_b200.install_as_ziggy()`: the reference's OWN model classes
     (`ziggy.hipgp.MeanFieldToeplitzGP`, `BlockToeplitzGP`) and `toeplitz_expanded.gram_solve` callers then run on top of the
@@ -22,7 +24,20 @@ import shutil
 import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-SRC = os.environ.get("HIPGP_REFERENCE_ROOT", "/root/reference")
+
+
+def reference_source():
+    """The reference checkout: $HIPGP_REFERENCE_ROOT, else BASELINE.json's reference_path (None if neither is given)."""
+    if os.environ.get("HIPGP_REFERENCE_ROOT"):
+        return os.environ["HIPGP_REFERENCE_ROOT"]
+    try:
+        with open(os.path.join(HERE, "..", "BASELINE.json")) as f:
+            return json.load(f).get("reference_path")
+    except (OSError, ValueError):
+        return None
+
+
+SRC = reference_source()
 DST = os.path.join(HERE, "_ref")
 FILES_EXTRA = ["experiments-hip-gp/run_solve_kn_experiment.py"]
 
@@ -35,8 +50,8 @@ def _sha(path):
 
 
 def stage(verbose=True):
-    """Returns the staged root, or None when the reference tree is not available (e.g. on the GPU box)."""
-    if not os.path.isdir(os.path.join(SRC, "ziggy")):
+    """Returns the staged root, or None when the reference tree is not available."""
+    if not SRC or not os.path.isdir(os.path.join(SRC, "ziggy")):
         return DST if os.path.isdir(os.path.join(DST, "ziggy")) else None
     manifest = {}
     pairs = []
@@ -71,6 +86,6 @@ def verify():
 if __name__ == "__main__":
     root = stage()
     if root is None:
-        print("reference tree not found at", SRC)
+        print("reference tree not found at %r (HIPGP_REFERENCE_ROOT or BASELINE.json reference_path)" % SRC)
         sys.exit(1)
     assert not verify()

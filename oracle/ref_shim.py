@@ -1,10 +1,10 @@
-"""Legacy-API shim that lets the UNMODIFIED reference (`/root/reference/ziggy`, pinned to
+"""Legacy-API shim that lets the UNMODIFIED reference (the `ziggy` package of suyashk12/hipgp, pinned to
 torch 1.4) import and run on torch >= 2.x.  TEST INFRASTRUCTURE ONLY.
 
 Used by `tests/golden/make_golden.py` (to generate the committed golden vectors, in the build container), by
 `tests/test_oracle_vs_reference.py` / `tests/test_gpu_dropin.py` and by `bench.py --impl reference`.  The reference is
-taken from `/root/reference` when that exists (build container) and otherwise from the staged, git-ignored, byte-identical
-copy `oracle/_ref/` written by `oracle/make_ref.py` (which is what travels to the GPU box); tests skip when neither is
+taken from the reference checkout (oracle/make_ref.py: $HIPGP_REFERENCE_ROOT, else BASELINE.json's reference_path) when
+that exists and otherwise from the staged, git-ignored, byte-identical copy `oracle/_ref/` written by `oracle/make_ref.py`; tests skip when neither is
 there.  Nothing in `hipgp_b200/` may import this module.
 
 What it patches (all removed from torch after 1.7):
@@ -27,14 +27,12 @@ _STAGED = _os.path.join(_os.path.dirname(_os.path.abspath(__file__)), "_ref")
 
 
 def reference_root():
-    """Directory that holds the unmodified `ziggy` package: /root/reference, else the staged copy oracle/_ref, else None."""
-    for root in ("/root/reference", _STAGED):
-        if _os.path.isdir(_os.path.join(root, "ziggy")):
+    """Directory that holds the unmodified `ziggy` package: the reference checkout, else the staged copy oracle/_ref, else None."""
+    from . import make_ref
+    for root in (make_ref.SRC, _STAGED):
+        if root and _os.path.isdir(_os.path.join(root, "ziggy")):
             return root
     return None
-
-
-REFERENCE_ROOT = reference_root() or "/root/reference"
 
 
 class _CallableFFTModule(types.ModuleType):
@@ -75,10 +73,10 @@ def install():
 
 
 def import_reference():
-    """Returns the unmodified reference package `ziggy` (raises if /root/reference is absent)."""
+    """Returns the unmodified reference package `ziggy` (raises if no reference tree is found)."""
     root = reference_root()
     if root is None:
-        raise ImportError("reference tree not present (neither /root/reference nor oracle/_ref; run oracle/make_ref.py)")
+        raise ImportError("reference tree not present (neither the reference checkout nor oracle/_ref; run oracle/make_ref.py)")
     install()
     if root not in sys.path:
         sys.path.insert(0, root)

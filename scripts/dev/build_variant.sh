@@ -2,7 +2,7 @@
 # usage: build_variant.sh <suffix> <extra nvcc flags...>   -- DEV_SMALL build of libhipgp_b200.so into hipgp_b200/csrc/variants/lib_<suffix>.so
 set -e
 SUF=$1; shift
-cd /root/repo/hipgp_b200/csrc
+cd "$(dirname "$0")/../../hipgp_b200/csrc"
 mkdir -p variants build/v_$SUF
 FLAGS="-gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -Xcompiler -fPIC $@"
 nvcc $FLAGS -c plan.cu -o build/v_$SUF/plan.o &

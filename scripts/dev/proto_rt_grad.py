@@ -1,5 +1,5 @@
-import numpy as np, torch, sys
-sys.path.insert(0,'/root/repo')
+import numpy as np, torch, sys, os
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), '..', '..'))
 torch.manual_seed(0)
 dt=torch.float64
 def embed(c):  # even extension per dim

@@ -1,6 +1,6 @@
 """Generates the committed golden vectors under tests/golden/ by running the UNMODIFIED reference
-(/root/reference/ziggy) under oracle/ref_shim.py.  Runs only in the build container (the reference tree
-does not travel to the GPU box).  Re-run with:  python tests/golden/make_golden.py
+(<checkout>/ziggy) under oracle/ref_shim.py.  Runs only where a reference checkout is available (it is not part of
+this repository).  Re-run with:  python tests/golden/make_golden.py  (checkout located as in oracle/make_ref.py)
 
 Every array here is an output of reference code on seeded inputs; nothing is produced by this repo's
 own implementation.  Files:

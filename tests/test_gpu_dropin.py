@@ -1,8 +1,8 @@
 """The UNMODIFIED reference running on top of the CUDA drop-ins (SURVEY.md section 8b: "the ziggy Python API stays a drop-in").
 
 `hipgp_b200.install_as_ziggy()` registers this package's modules under the reference's module names; the reference's OWN
-callers are then imported from the staged copy `oracle/_ref/ziggy` (oracle/make_ref.py; byte-identical to /root/reference,
-git-ignored, ships to the GPU box like the built .so):
+callers are then imported from the staged copy `oracle/_ref/ziggy` (oracle/make_ref.py; byte-identical to the reference
+checkout, git-ignored; skipped where it is not staged):
 
   * `ziggy.hipgp.MeanFieldToeplitzGP` / `BlockToeplitzGP` (hipgp.py:449-690): `elbo_and_grad` + `predict` against the golden
     vectors generated from the reference running on its own torch implementation (tests/golden/make_golden.py);
@@ -160,7 +160,7 @@ print("DROPIN_OK")
 
 def _run(script):
     if not os.path.isdir(os.path.join(REF, "ziggy")):
-        pytest.skip("oracle/_ref not staged (python oracle/make_ref.py in the build container)")
+        pytest.skip("oracle/_ref not staged: needs the reference checkout (python oracle/make_ref.py)")
     r = subprocess.run([sys.executable, "-c", script % {"root": ROOT, "ref": REF}], capture_output=True, text=True, timeout=900)
     assert r.returncode == 0 and "DROPIN_OK" in r.stdout, r.stdout[-3000:] + r.stderr[-6000:]
 
