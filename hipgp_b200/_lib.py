@@ -51,6 +51,7 @@ SIGNATURES = {
     "hipgp_meanfield_colstats": (_i, [_i, _vp, _vp, _vp, _i64, _i64, _vp, _vp, _vp]),
     "hipgp_block_lam": (_i, [_i, _vp, _vp, _vp, _i64, _i64, _i64, _i64, _d, _d, _vp, _vp]),
     "hipgp_block_diag_multiply": (_i, [_i, _vp, _vp, _vp, _i64, _i64, _i64, _i64, _vp, _vp]),
+    "hipgp_block_quadform_grad": (_i, [_i, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _i64, _vp, _vp]),
     "hipgp_toeplitz_quadform": (_i, [_vp, _vp, _vp, _i64, _d, _vp, _vp]),
     "hipgp_rt_column_grad": (_i, [_vp, _vp, _vp, _i64, _d, _vp, _vp]),
     "hipgp_plan_set_slab": (_i, [_vp, _i, _i]),

@@ -14,7 +14,7 @@ from torch import nn
 from .toeplitz_tensor import ToeplitzTensor
 from . import kernels as hk
 from . import dist as hdist
-from .plan import meanfield_rowstats, meanfield_colstats, block_lam, block_diag_multiply, row_dot
+from .plan import meanfield_rowstats, meanfield_colstats, block_lam, block_diag_multiply, block_quadform_grad, row_dot
 from . import util as hutil
 
 
@@ -323,12 +323,34 @@ class MeanFieldToeplitzGP(ToeplitzInducingGP):
         return knt_m[:, None].cpu().detach(), sig_star.cpu().detach()
 
 
+class _BlockKnSkn(torch.autograd.Function):
+    """knSkn_b = kn_b^T blockdiag(S) kn_b for kn (B, M'), S (num_blocks, bs, bs) read through the block index map, as a
+    differentiable map (the reference gets its gradient from autograd through block_diag_multiply, hipgp.py:640-652).
+    Forward: compute_knSkn's kernels.  Backward: dkn = g (S + S^T) kn through `hipgp_block_quadform_grad`, and, when S
+    requires a gradient (`elbo` in the 'standard' parameterisation), dS_k = sum_b g_b kn_blk,b kn_blk,b^T through
+    `hipgp_block_lam`."""
+
+    @staticmethod
+    def forward(ctx, kn, S, blk_idx):
+        ctx.save_for_backward(kn, S, blk_idx)
+        return row_dot(kn, block_diag_multiply(S, kn, blk_idx))
+
+    @staticmethod
+    def backward(ctx, grad_output):
+        kn, S, idx = ctx.saved_tensors
+        g = grad_output.contiguous()
+        dkn = block_quadform_grad(S, kn, g, idx) if ctx.needs_input_grad[0] else None
+        dS = block_lam(kn, g, idx, scale=1.0, diag=0.0).to(S.dtype) if ctx.needs_input_grad[1] else None
+        return dkn, dS, None
+
+
 class BlockToeplitzGP(MeanFieldToeplitzGP):
     """Block-diagonal variational family (ziggy/hipgp.py:527-690): q(u) = N(m, blockdiag(S_k)) with the blocks being
     neighbouring chunks of the WHITENED (2m-2)-grid.  `qm` is kept in Toeplitz ordering, the blocks in block ordering;
     the two contractions over k_n run through `hipgp_block_lam` / `hipgp_block_diag_multiply`, which read k_n through the
     index map (no permuted copies, no (bsz, num_blocks, bs, bs) outer products as in hipgp.py:252-255).  The ELBO /
-    natural-gradient step and `predict` are the shared code of the mean-field class with this family's statistics."""
+    natural-gradient step and `predict` are the shared code of the mean-field class with this family's statistics;
+    learn_kernel / learn_noise take the mean-field class's traced step with knSkn through `_BlockKnSkn`."""
 
     def __init__(self, kernel, xgrids, num_obs, xblock_size=10, block_sizes=None, sig2_init=1., ell_init=.05, noise2_init=1.,
                  init_Svar=.1, learn_kernel=False, learn_noise=False, dtype=torch.float, whitened_type='ziggy',
@@ -336,9 +358,6 @@ class BlockToeplitzGP(MeanFieldToeplitzGP):
         ToeplitzInducingGP.__init__(self, kernel, xgrids, num_obs, sig2_init=sig2_init, ell_init=ell_init,
                                     noise2_init=noise2_init, learn_kernel=learn_kernel, learn_noise=learn_noise, dtype=dtype,
                                     whitened_type=whitened_type, parameterization=parameterization, jitter_val=jitter_val)
-        if learn_kernel or learn_noise:
-            raise NotImplementedError("hipgp_b200.BlockToeplitzGP: hyper-parameter learning (learn_kernel / learn_noise) is wired for the "
-                                      "mean-field family only; the block family keeps its kernel parameters fixed")
         input_dim = len(xgrids)
         if block_sizes is not None:
             assert input_dim == len(block_sizes), "xgrids ndim = {}, block ndim = {}".format(input_dim, len(block_sizes))
@@ -399,6 +418,10 @@ class BlockToeplitzGP(MeanFieldToeplitzGP):
 
     def compute_knSkn(self, kn, qS):
         return row_dot(kn, self.block_diag_multiply(qS, kn))
+
+    def _knSkn_traced(self, kn, qS):
+        """knSkn on the autograd tape (compute_batch_an under learn_kernel / learn_noise, and `elbo`)"""
+        return _BlockKnSkn.apply(kn, qS, self._idx(kn.device))
 
     def get_identity_for_lam(self):
         return torch.eye(self.block_size, device=self.xgrids[0].device, dtype=self.dtype)

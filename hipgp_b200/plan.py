@@ -315,6 +315,27 @@ def block_diag_multiply(S_block, v, blk_idx):
     return out
 
 
+def block_quadform_grad(S_block, kn, g, blk_idx):
+    """g[:, None] * from_blocks((S_block + S_block^T) @ to_blocks(kn)): the gradient of knSkn_b = kn_b^T blockdiag(S) kn_b
+    with upstream g (B,), in one pass over kn and S.  Returns (B, M')."""
+    _require_cuda(kn, "kn")
+    lib = L.load()
+    kn = kn.contiguous(); S = S_block.to(kn.dtype).contiguous(); g = g.reshape(-1).to(kn.dtype).contiguous()
+    idx = _blk_idx(blk_idx, kn.device)
+    B, E = kn.shape
+    nblk, bs = idx.shape
+    if tuple(S.shape) != (nblk, bs, bs):
+        raise ValueError("S_block must be (num_blocks, block_size, block_size)")
+    if g.numel() != B:
+        raise ValueError("g must have one entry per row of kn")
+    out = torch.empty_like(kn)
+    with torch.cuda.device(kn.device):
+        L.check(lib, lib.hipgp_block_quadform_grad(_DT[kn.dtype], C.c_void_p(S.data_ptr()), C.c_void_p(kn.data_ptr()),
+                                                   C.c_void_p(g.data_ptr()), C.c_void_p(idx.data_ptr()), B, E, nblk, bs,
+                                                   C.c_void_p(out.data_ptr()), _stream_ptr(kn.device)))
+    return out
+
+
 def row_dot(a, b):
     """per-row dot products of two (B, M) tensors, deterministic fixed-order reduction (hipgp_vec_dot).  Returns (B,)."""
     _require_cuda(a, "a")

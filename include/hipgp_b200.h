@@ -155,6 +155,14 @@ int hipgp_block_lam(int dtype, const void* kn_dev, const void* w_dev, const int6
                     int64_t nblk, int64_t bs, double scale, double diag, void* lam_dev, void* stream);
 int hipgp_block_diag_multiply(int dtype, const void* S_dev, const void* v_dev, const int64_t* blk_idx_dev, int64_t B,
                               int64_t E, int64_t nblk, int64_t bs, void* out_dev, void* stream);
+/* block_quadform_grad:  dkn[b, idx[k,i]] = g[b] sum_j (S[k][i][j] + S[k][j][i]) kn[b, idx[k,j]]
+ *                       the gradient of knSkn_b = kn_b^T blockdiag(S) kn_b with upstream g (B), which the reference gets from
+ *                       autograd through block_diag_multiply and the row sum of compute_batch_an (hipgp.py:640-652, :370-414)
+ *                       when it traces kernel / noise hyper-parameters (:214-218).  S + S^T, so any S (the 'standard'
+ *                       parameterisation does not keep it symmetric).  Deterministic (no atomics); B = 0 is a no-op;
+ *                       dkn must not overlap kn. */
+int hipgp_block_quadform_grad(int dtype, const void* S_dev, const void* kn_dev, const void* g_dev, const int64_t* blk_idx_dev,
+                              int64_t B, int64_t E, int64_t nblk, int64_t bs, void* dkn_dev, void* stream);
 
 /* ---- Toeplitz-column quadratic form: the kernel-hyper-parameter gradient of InvMatmul.backward
  * (ziggy/misc/_inv_matmul.py:39-55 -> gpt_toeplitz.py:169-209 sym_toeplitz_derivative_quadratic_form, evaluated there on
