@@ -47,6 +47,7 @@ SIGNATURES = {
     "hipgp_kernel_pairwise": (_i, [_i, _i, _i, _d, _pd, _i, _d, _vp, _i64, _vp, _i64, _i, _vp, _i, _vp, _vp]),
     "hipgp_kxu_param_grad": (_i, [_i, _i, _i, _d, _pd, _i, _vp, _i64, _i, _pi64, _vp, _vp, _i64, _vp, _i, _vp, _vp, _vp]),
     "hipgp_doubly_diag": (_i, [_i, _vp, _i64, _i, _d, _pd, _i, _vp, _vp, _vp, _i, _vp, _vp]),
+    "hipgp_doubly_diag_param_grad": (_i, [_i, _vp, _i64, _i, _d, _pd, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp]),
     "hipgp_meanfield_rowstats": (_i, [_i, _vp, _vp, _vp, _i64, _i64, _vp, _vp]),
     "hipgp_meanfield_colstats": (_i, [_i, _vp, _vp, _vp, _i64, _i64, _vp, _vp, _vp]),
     "hipgp_block_lam": (_i, [_i, _vp, _vp, _vp, _i64, _i64, _i64, _i64, _d, _d, _vp, _vp]),

@@ -140,6 +140,22 @@ __global__ void __launch_bounds__(256) kxu_kernel(KxuParams P, const T* __restri
     }
 }
 
+// The table interval of KernelDoublyDiagInterpolator.forward (kernels.py:205-207) for observation b: the scaled distance
+// |x_b / ell| and the index of the last table distance below it.
+template <class T>
+__device__ __forceinline__ int doubly_diag_lookup(const T* __restrict__ xb, long b, int ndim, const T* ell, const T* __restrict__ dgrid,
+                                                  int ntab, T* dist_out) {
+    T sq = 0;
+    for (int d = 0; d < ndim; ++d) { const T t = xb[b * ndim + d] / ell[d]; sq += t * t; }
+    const T dist = M_<T>::sqrt(sq);
+    int cnt = 0;
+    for (int t = 0; t < ntab; ++t) cnt += (dist > dgrid[t]) ? 1 : 0;
+    int li = cnt - 1;
+    if (li < 0) li += ntab;                 // python negative index wraps to the last entry (SURVEY 8a-bis)
+    *dist_out = dist;
+    return li;
+}
+
 // KernelDoublyDiagInterpolator.forward, kernels.py:199-218
 template <class T>
 __global__ void doubly_diag_kernel(const T* __restrict__ xb, long B, int ndim, double sig2, double ell0,
@@ -148,13 +164,8 @@ __global__ void doubly_diag_kernel(const T* __restrict__ xb, long B, int ndim, d
     const long b = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= B) return;
     const T ell[3] = {(T)e0, (T)e1, (T)e2};
-    T sq = 0;
-    for (int d = 0; d < ndim; ++d) { const T t = xb[b * ndim + d] / ell[d]; sq += t * t; }
-    const T dist = M_<T>::sqrt(sq);
-    int cnt = 0;
-    for (int t = 0; t < ntab; ++t) cnt += (dist > dgrid[t]) ? 1 : 0;
-    int li = cnt - 1;
-    if (li < 0) li += ntab;                 // python negative index wraps to the last entry (SURVEY 8a-bis)
+    T dist;
+    const int li = doubly_diag_lookup<T>(xb, b, ndim, ell, dgrid, ntab, &dist);
     const T diff = dist - dgrid[li];
     const T iv = knn[li] + slopes[li] * diff;
     out[b] = (T)ell0 * (T)ell0 * (T)sig2 * iv;
@@ -203,7 +214,12 @@ __device__ __forceinline__ void eval_point_grad(const KxuParams& P, const T* x, 
 }
 
 // partial[(b * gridDim.x + blockIdx.x) * 4 + {0, 1, 2, 3}] = sum over this block's columns of G[b][j] * {dk/dsig2, dk/dell_0..2}
-// (modes POINT and SEMI_MC; grid as kxu_kernel)
+// (modes POINT, SEMI_ANALYTIC and SEMI_MC; grid as kxu_kernel)
+//
+// SEMI_ANALYTIC (SqExp, kernels.py:223-237): k = sig2 |x| I0 with I_k = int_0^1 alpha^k e(alpha) dalpha,
+// e(alpha) = exp(-(a alpha^2 - 2 b alpha + c) / 2), a = x^T S x, b = x^T S u, c = u^T S u, S = diag(1 / ell_d^2).
+// Integration by parts (e' = -(a alpha - b) e) gives I1 = (b I0 + e(0) - e(1)) / a and I2 = (b I1 + I0 - e(1)) / a, so
+// dk/dsig2 = |x| I0 and dk/dell_d = sig2 |x| / ell_d^3 (x_d^2 I2 - 2 x_d u_d I1 + u_d^2 I0).
 template <class T>
 __global__ void __launch_bounds__(256) kxu_grad_kernel(KxuParams P, const T* __restrict__ xb, const T* __restrict__ grids,
                                                        const T* __restrict__ ypts, const T* __restrict__ alphas,
@@ -228,6 +244,27 @@ __global__ void __launch_bounds__(256) kxu_grad_kernel(KxuParams P, const T* __r
         if (P.mode == 0) {
             eval_point_grad<T>(P, x, u, &ds, de);
             acc[0] += g * ds; acc[1] += g * de[0]; acc[2] += g * de[1]; acc[3] += g * de[2];
+        } else if (P.mode == 1) {
+            double a = 0, bq = 0, c = 0;
+            for (int d = 0; d < P.ndim; ++d) {
+                const double xd = (double)x[d], ud = (double)u[d], si = 1.0 / (P.ell[d] * P.ell[d]);
+                a += xd * si * xd; bq += xd * si * ud; c += ud * si * ud;
+            }
+            const double r2a = ::sqrt(2.0 * a);
+            const double I0 = ::exp(bq * bq / (2.0 * a) - 0.5 * c) * ::sqrt(1.5707963267948966 / a) *
+                              (::erf((a - bq) / r2a) - ::erf(-bq / r2a));
+            const double e0 = ::exp(-0.5 * c), e1 = ::exp(-0.5 * (a - 2.0 * bq + c));
+            const double I1 = (bq * I0 + e0 - e1) / a;
+            const double I2 = (bq * I1 + I0 - e1) / a;
+            acc[0] += g * xnorm * I0;
+            const double f = g * P.sig2 * xnorm;
+#pragma unroll
+            for (int d = 0; d < 3; ++d) {
+                if (d < P.ndim) {
+                    const double xd = (double)x[d], ud = (double)u[d], el = P.ell[d];
+                    acc[1 + d] += f / (el * el * el) * (xd * xd * I2 - 2.0 * xd * ud * I1 + ud * ud * I0);
+                }
+            }
         } else {          // SEMI_MC: mean over the stratified points alpha_t x, times |x|
             double s0 = 0, s1 = 0, s2 = 0, s3 = 0;
             for (int t = 0; t < P.npts; ++t) {
@@ -245,6 +282,31 @@ __global__ void __launch_bounds__(256) kxu_grad_kernel(KxuParams P, const T* __r
         const double t = block_sum_256<T>(acc[c]);
         if (threadIdx.x == 0) partial[((size_t)b * gridDim.x + blockIdx.x) * 4 + c] = t;
     }
+}
+
+// Backward of doubly_diag_kernel for a scalar ell: out_b = ell^2 sig2 iv_b with iv_b = knn[i] + slopes[i] (dist_b - dgrid[i]) and
+// dist_b = |x_b| / ell, so d out_b / d sig2 = ell^2 iv_b and d out_b / d ell = sig2 ell (2 iv_b - slopes[i] dist_b).
+// grid ceil(B / 256), block 256: partial[blockIdx.x * 2 + {0, 1}] = this block's sums of g_b * {d/dsig2, d/dell}.
+template <class T>
+__global__ void __launch_bounds__(256) doubly_diag_grad_kernel(const T* __restrict__ xb, long B, int ndim, double sig2, double ell0,
+                                                               const T* __restrict__ dgrid, const T* __restrict__ slopes,
+                                                               const T* __restrict__ knn, int ntab, const T* __restrict__ g,
+                                                               double* __restrict__ partial) {
+    const long b = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    double ds = 0, de = 0;
+    if (b < B) {
+        const T ell[3] = {(T)ell0, (T)ell0, (T)ell0};
+        T dist;
+        const int li = doubly_diag_lookup<T>(xb, b, ndim, ell, dgrid, ntab, &dist);
+        const double sl = (double)slopes[li];
+        const double iv = (double)knn[li] + sl * ((double)dist - (double)dgrid[li]);
+        const double gb = (double)g[b];
+        ds = gb * ell0 * ell0 * iv;
+        de = gb * sig2 * ell0 * (2.0 * iv - sl * (double)dist);
+    }
+    ds = block_sum_256<T>(ds);
+    de = block_sum_256<T>(de);
+    if (threadIdx.x == 0) { partial[(size_t)blockIdx.x * 2] = ds; partial[(size_t)blockIdx.x * 2 + 1] = de; }
 }
 
 // grid (nchunk, B), block 256; op 0: dot(a,b) | op 1: x += al p, r -= al Ap, dot(r,r) | op 2: p = z + be p

@@ -94,9 +94,10 @@ def _with_param_grad(call, params, meta):
     sig2, ell = params
     if not _wants_grad(sig2, ell):
         return call(params)
-    if meta["kernel_id"] == L.K_GNEITING or meta["mode"] not in (L.KXU_POINT, L.KXU_SEMI_MC):
+    if meta["kernel_id"] == L.K_GNEITING or meta["mode"] not in (L.KXU_POINT, L.KXU_SEMI_ANALYTIC, L.KXU_SEMI_MC):
         raise NotImplementedError("hipgp_b200: hyper-parameter gradients (learn_kernel=True) are built for the SqExp / Matern point "
-                                  "kernels and their Monte-Carlo line integrals; not for this kernel / estimator")
+                                  "kernels, their Monte-Carlo line integrals and the analytic SqExp line integral; not for this "
+                                  "kernel / estimator")
     dev = meta["x"].device
     s_t = sig2 if isinstance(sig2, torch.Tensor) else torch.tensor(float(sig2), dtype=torch.float64, device=dev)
     e_t = ell if isinstance(ell, torch.Tensor) else torch.tensor(np.asarray(ell, dtype=np.float64), device=dev)
@@ -344,11 +345,49 @@ class KernelDoublyDiagInterpolator(nn.Module):
         sl = self.slopes.to(x.device).contiguous()
         kn = self.knn.to(x.device).contiguous()
         ellv, n_ell = _ell_array(ell, D)
-        out = torch.empty(n, dtype=self.dtype, device=x.device)
-        with torch.cuda.device(x.device):
-            L.check(lib, lib.hipgp_doubly_diag(_DT[self.dtype], _ptr(x), n, D, _f(sig2), ellv, n_ell, _ptr(dg), _ptr(sl),
-                                               _ptr(kn), dg.numel(), _ptr(out), _stream(x.device)))
-        return out
+        dt = _DT[self.dtype]
+
+        def call():
+            out = torch.empty(n, dtype=self.dtype, device=x.device)
+            with torch.cuda.device(x.device):
+                L.check(lib, lib.hipgp_doubly_diag(dt, _ptr(x), n, D, _f(sig2), ellv, n_ell, _ptr(dg), _ptr(sl), _ptr(kn), dg.numel(),
+                                                   _ptr(out), _stream(x.device)))
+            return out
+        if not _wants_grad(sig2, ell):
+            return call()
+        if n_ell != 1:
+            raise NotImplementedError("hipgp_b200: hyper-parameter gradients of the doubly integrated diagonal need a scalar ell "
+                                      "(the prefactor ell^2 is not defined for a per-axis ell)")
+
+        def grad_call(g):
+            g = g.to(self.dtype).contiguous()
+            partial = torch.empty(((n + 255) // 256, 2), dtype=torch.float64, device=x.device)
+            with torch.cuda.device(x.device):
+                L.check(lib, lib.hipgp_doubly_diag_param_grad(dt, _ptr(x), n, D, _f(sig2), ellv, n_ell, _ptr(dg), _ptr(sl), _ptr(kn),
+                                                              dg.numel(), _ptr(g), _ptr(partial), _stream(x.device)))
+            return partial.sum(dim=0)
+        s_t = sig2 if isinstance(sig2, torch.Tensor) else torch.tensor(float(sig2), dtype=torch.float64, device=x.device)
+        e_t = ell if isinstance(ell, torch.Tensor) else torch.tensor(float(ell), dtype=torch.float64, device=x.device)
+        return _DoublyDiagParamGrad.apply(s_t, e_t, call, grad_call)
+
+
+class _DoublyDiagParamGrad(torch.autograd.Function):
+    """The doubly integrated diagonal as a differentiable function of (sig2, ell) for a scalar ell: the forward is the
+    hipgp_doubly_diag call of the no-grad path, the backward reduces g * d/d(sig2, ell) in hipgp_doubly_diag_param_grad.
+    learn_kernel=True in the reference differentiates kernels.py:199-218 with autograd."""
+
+    @staticmethod
+    def forward(ctx, sig2_t, ell_t, call, grad_call):
+        ctx.grad_call = grad_call
+        ctx.sig2_dtype, ctx.ell_dtype, ctx.ell_shape = sig2_t.dtype, ell_t.dtype, ell_t.shape
+        return call()
+
+    @staticmethod
+    def backward(ctx, g):
+        tot = ctx.grad_call(g)
+        g_sig2 = tot[0].to(ctx.sig2_dtype).reshape(()) if ctx.needs_input_grad[0] else None
+        g_ell = tot[1].to(ctx.ell_dtype).reshape(ctx.ell_shape) if ctx.needs_input_grad[1] else None
+        return g_sig2, g_ell, None, None
 
 
 # --------------------------------------------------------------------------------------------------

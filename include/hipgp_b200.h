@@ -128,7 +128,8 @@ int hipgp_kernel_pairwise(int dtype, int kernel_id, int mode, double sig2, const
 /* hyper-parameter derivatives of K_xu for learn_kernel=True (the reference lets autograd differentiate kernels.py:73-79,
  * 145-158): per-block partial sums of G * {dk/dsig2, dk/dell_0, dk/dell_1, dk/dell_2} over the columns of row b; `partial` holds
  * B * ceil(M/1024) * 4 doubles, the caller adds them up.  Either the 1-D grids (grids != NULL, as hipgp_kxu) or an explicit
- * second point set ypts (n_y x ndim, as hipgp_kernel_pairwise).  Modes POINT and SEMI_MC; SqExp / Matern kernels. */
+ * second point set ypts (n_y x ndim, as hipgp_kernel_pairwise).  Modes POINT and SEMI_MC with the SqExp / Matern kernels;
+ * SEMI_ANALYTIC with SqExp (closed form of the derivative of the analytic line integral). */
 int hipgp_kxu_param_grad(int dtype, int kernel_id, int mode, double sig2, const double* ell, int n_ell, const void* x_dev, int64_t B,
                          int ndim, const int64_t* m, const void* grids_dev, const void* ypts_dev, int64_t n_y, const void* mc_alphas_dev,
                          int npts, const void* G_dev, double* partial_dev, void* stream);
@@ -136,6 +137,13 @@ int hipgp_kxu_param_grad(int dtype, int kernel_id, int mode, double sig2, const 
 int hipgp_doubly_diag(int dtype, const void* x_dev, int64_t B, int ndim, double sig2, const double* ell, int n_ell,
                       const void* distance_grid_dev, const void* slopes_dev, const void* knn_dev, int ntab,
                       void* out_dev, void* stream);
+/* hyper-parameter derivatives of hipgp_doubly_diag for learn_kernel=True (the reference lets autograd differentiate
+ * kernels.py:199-218): with out_b = ell^2 sig2 iv_b, d/dsig2 = ell^2 iv_b and d/dell = sig2 ell (2 iv_b - slope_b |x_b| / ell).
+ * Scalar ell only (n_ell == 1).  g: upstream gradient (B, dtype).  partial holds ceil(B/256) * 2 doubles = per-block sums of
+ * g * {d/dsig2, d/dell}; the caller adds them up.  B = 0 is a no-op. */
+int hipgp_doubly_diag_param_grad(int dtype, const void* x_dev, int64_t B, int ndim, double sig2, const double* ell, int n_ell,
+                                 const void* distance_grid_dev, const void* slopes_dev, const void* knn_dev, int ntab,
+                                 const void* g_dev, double* partial_dev, void* stream);
 
 /* ---- mean-field natural-gradient reductions over k_n (B, M') (ziggy/hipgp.py:241-250,395-397,439,524).
  * rowstats: out[0][b] = k_n[b].qm, out[1][b] = k_n[b].k_n[b], out[2][b] = sum_j k_n[b,j]^2 qS[j]   (3 x B, plan dtype)
