@@ -56,10 +56,6 @@ SIGNATURES = {
     "hipgp_toeplitz_quadform": (_i, [_vp, _vp, _vp, _i64, _d, _vp, _vp]),
     "hipgp_rt_column_grad": (_i, [_vp, _vp, _vp, _i64, _d, _vp, _vp]),
     "hipgp_plan_set_slab": (_i, [_vp, _i, _i]),
-    "hipgp_slab_sizes": (_i, [_vp, _pi64, _pi64]),
-    "hipgp_slab_stage1": (_i, [_vp, _vp, _vp, _vp]),
-    "hipgp_slab_stage2": (_i, [_vp, _i, _vp, _vp]),
-    "hipgp_slab_stage3": (_i, [_vp, _vp, _vp, _vp]),
     "hipgp_slab2_sizes": (_i, [_vp, _pi64, _pi64]),
     "hipgp_slab2_stage_a": (_i, [_vp, _vp, _vp, _vp]),
     "hipgp_slab2_stage_b": (_i, [_vp, _i, _vp, _vp]),

@@ -322,7 +322,7 @@ __global__ void __launch_bounds__(NT, MINB) cols_blk_kernel(const HIPGP_GRID_CON
                 Lane<T>* base = s + (G::slot(p0) * NL + lane);
                 Lane<T> v[RLAST];
                 if (mode == CM_INV) {
-                    const cplx<T>* gp = in + cols_rowoff<T>(p0, P.pitch, P.in_split_len, P.in_split_stride) + lane * LPT;
+                    const cplx<T>* gp = in + (size_t)p0 * P.pitch + lane * LPT;
 #pragma unroll
                     for (int r = 0; r < RLAST; ++r) v[r] = ok ? lane_from_global(gp + r * pitch) : lzero<T>();
                 } else {
@@ -343,7 +343,7 @@ __global__ void __launch_bounds__(NT, MINB) cols_blk_kernel(const HIPGP_GRID_CON
                 }
                 if (mode == CM_FWD) {
                     if (ok) {
-                        cplx<T>* gp = out + cols_rowoff<T>(p0, P.pitch, P.out_split_len, P.out_split_stride) + lane * LPT;
+                        cplx<T>* gp = out + (size_t)p0 * P.pitch + lane * LPT;
 #pragma unroll
                         for (int r = 0; r < RLAST; ++r) lane_to_global(gp + r * pitch, v[r]);
                     }

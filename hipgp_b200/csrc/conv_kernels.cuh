@@ -127,8 +127,8 @@ struct RowsParams {
     int mode, dot_kind, do_fft;
     int vec_ok;           // all row pointers are aligned for 2-element vector access
     int vec16_ok;         // ... and for 16-byte access (specialised kernels stream rows in 16-byte chunks)
-    int tma_ok;           // specialised kernels: row blocks move with 1-D bulk-asynchronous (TMA) copies
-    int tma_op;           // ... including the operands of a fused PCG update (they land in the idle tile buffer, which is big enough)
+    int tma_op;           // specialised kernels move aligned row blocks with 1-D bulk-asynchronous (TMA) copies; 1 = so do the
+                          // operands of a fused PCG update (they land in the idle tile buffer, which is big enough)
     const void* spec; int spec_kind;   // rows_inv only (1-D grids)
     PcgDev st;
 };
@@ -332,14 +332,7 @@ struct ColsParams {
     int tma_spec;                 // ... and the real spectrum tile as ONE padded TMA box
     int batch_fastest;            // ... walked batch-fastest (big spectra: a spectrum tile is reused by the CTAs running side by side)
     const int* done_flag;         // optional PCG early-exit flag
-    // slab-decomposed grids: rows of the output (FWD) / input (INV) are scattered / gathered in blocks of `split_len`
-    // positions, `split_stride` elements apart, so that the pass writes (reads) the all-to-all buffer directly
-    int out_split_len; long out_split_stride;
-    int in_split_len; long in_split_stride;
 };
-template <class T> __device__ __forceinline__ size_t cols_rowoff(int i, long pitch, int split_len, long split_stride) {
-    return split_len ? (size_t)(i / split_len) * split_stride + (size_t)(i % split_len) * pitch : (size_t)i * pitch;
-}
 
 template <class T>
 __global__ void __launch_bounds__(512) cols_pass_kernel(ColsParams<T> P) {
@@ -357,7 +350,7 @@ __global__ void __launch_bounds__(512) cols_pass_kernel(ColsParams<T> P) {
     for (int w = tid; w < L * TB; w += nthreads) {
         const int c = w % TB, i = w / TB;
         cplx<T> v = mk<T>(0, 0);
-        if (i < rows_in && c < nc) v = in[cols_rowoff<T>(i, P.pitch, P.in_split_len, P.in_split_stride) + c];
+        if (i < rows_in && c < nc) v = in[(size_t)i * P.pitch + c];
         s[(size_t)i * TBP + c] = v;
     }
     __syncthreads();
@@ -375,7 +368,7 @@ __global__ void __launch_bounds__(512) cols_pass_kernel(ColsParams<T> P) {
     const int rows_out = P.mode == CM_FWD ? L : P.n_out;
     for (int w = tid; w < rows_out * TB; w += nthreads) {
         const int c = w % TB, i = w / TB;
-        if (c < nc) out[cols_rowoff<T>(i, P.pitch, P.out_split_len, P.out_split_stride) + c] = s[(size_t)i * TBP + c];
+        if (c < nc) out[(size_t)i * P.pitch + c] = s[(size_t)i * TBP + c];
     }
 }
 

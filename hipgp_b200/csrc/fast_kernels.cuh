@@ -104,7 +104,7 @@ __global__ void __launch_bounds__(NT, MINB) cols_fast_kernel(ColsParams<T> P) {
                 Lane<T> v[R0];
 #pragma unroll
                 for (int r = 0; r < R0; ++r)
-                    v[r] = r < rows_in ? lane_from_global(in + cols_rowoff<T>(r, P.pitch, P.in_split_len, P.in_split_stride) + lane * LPT) : lzero<T>();
+                    v[r] = r < rows_in ? lane_from_global(in + (size_t)r * P.pitch + lane * LPT) : lzero<T>();
                 if (mode != CM_INV) lbfly<R0, false, T>(v);
                 if (mode == CM_FUSED) {
 #pragma unroll
@@ -113,7 +113,7 @@ __global__ void __launch_bounds__(NT, MINB) cols_fast_kernel(ColsParams<T> P) {
                 if (mode != CM_FWD) lbfly<R0, true, T>(v);
 #pragma unroll
                 for (int r = 0; r < R0; ++r)
-                    if (r < rows_out) lane_to_global(out + cols_rowoff<T>(r, P.pitch, P.out_split_len, P.out_split_stride) + lane * LPT, v[r]);
+                    if (r < rows_out) lane_to_global(out + (size_t)r * P.pitch + lane * LPT, v[r]);
             }
         }
         return;
@@ -228,8 +228,7 @@ __global__ void __launch_bounds__(NT, MINB) cols_fast_kernel(ColsParams<T> P) {
                     Lane<T>* base = s + (G::slot(p0) * NL + lane);
                     Lane<T> v[RLAST];
                     if (mode == CM_INV) {
-                        // (slab grids: rows may be gathered in blocks of in_split_len positions, a multiple of RLAST)
-                        const cplx<T>* gp = in + cols_rowoff<T>(p0, P.pitch, P.in_split_len, P.in_split_stride) + lane * LPT;
+                        const cplx<T>* gp = in + (size_t)p0 * P.pitch + lane * LPT;
 #pragma unroll
                         for (int r = 0; r < RLAST; ++r) v[r] = ok ? lane_from_global(gp + r * pitch) : lzero<T>();
                     } else {
@@ -250,7 +249,7 @@ __global__ void __launch_bounds__(NT, MINB) cols_fast_kernel(ColsParams<T> P) {
                     }
                     if (mode == CM_FWD) {
                         if (ok) {
-                            cplx<T>* gp = out + cols_rowoff<T>(p0, P.pitch, P.out_split_len, P.out_split_stride) + lane * LPT;
+                            cplx<T>* gp = out + (size_t)p0 * P.pitch + lane * LPT;
 #pragma unroll
                             for (int r = 0; r < RLAST; ++r) lane_to_global(gp + r * pitch, v[r]);
                         }
@@ -346,7 +345,7 @@ __global__ void __launch_bounds__(NT, MINB) rows_fwd_fast_kernel(RowsParams<T> P
     // vector, no register staging; the update then runs shared memory -> shared memory and the updated vector leaves with
     // one bulk store.  Only x of the x/r update (read AND written) goes through ordinary 16-byte accesses.
     bool bulk_store_pending = false;
-    if (P.tma_ok && P.vec16_ok && SROW == n && (mode == RF_PLAIN || mode == RF_SELFDOT || P.tma_op)) {
+    if (P.vec16_ok && SROW == n && (mode == RF_PLAIN || mode == RF_SELFDOT || P.tma_op)) {
         constexpr int CH = 16 / (int)sizeof(T);
         __shared__ __align__(8) unsigned long long s_mbar;
         const unsigned bytes = (unsigned)((size_t)nl * n * sizeof(T));
@@ -872,7 +871,7 @@ __global__ void __launch_bounds__(NT, MINB) rows_inv_fast_kernel(RowsParams<T> P
         }
     }
 #ifndef HIPGP_EMU
-    const bool tma_any = P.tma_ok && P.vec16_ok && SROW == n;
+    const bool tma_any = P.vec16_ok && SROW == n;
     const bool tma_out = !want_dot && tma_any;
     const bool tma_dot = want_dot && tma_any;       // fused dot: the rows still leave with ONE bulk store; the warps only read
     if (tma_any) fence_proxy_async();        // this thread's shared-memory writes become visible to the async proxy

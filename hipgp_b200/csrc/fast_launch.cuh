@@ -66,11 +66,8 @@ static void launch_rows_fast_t(hipgp_plan* pl, bool inverse, RowsParams<T>& P, c
     // the tile, then the side buffer: the tile's real rows, row-major
     const size_t smem = G::smem_bytes() + sizeof(T) * (size_t)((P.n_real + 3) & ~3) * NROW;
     if (smem > 227 * 1024) throw Error("row pass: rows too long for the shared-memory side buffer");
-    static const char* env_nt = getenv("HIPGP_NO_TMA");
-    static const char* env_nf = getenv("HIPGP_NO_TMA_FUSED");
-    P.tma_ok = env_nt ? 0 : 1;
     // operands of a fused update land in the tile buffer: two row blocks must fit in it
-    P.tma_op = (!env_nf && !inverse && 2 * sizeof(T) * (size_t)((P.n_real + 3) & ~3) * NROW <= G::smem_bytes()) ? 1 : 0;
+    P.tma_op = (!inverse && 2 * sizeof(T) * (size_t)((P.n_real + 3) & ~3) * NROW <= G::smem_bytes()) ? 1 : 0;
     dim3 grid((unsigned)((P.total_rows + NROW - 1) / NROW));
     PROF_BEGIN(pl, inverse ? 2 : 0, st);
     if (inverse) {
@@ -109,14 +106,10 @@ static void launch_cols_fast_t(hipgp_plan* pl, ColsParams<T>& P, long n_outer, l
     static_assert(C::Ln == LEN, "radix list does not multiply to the length");
     constexpr int TBL = C::NLC * C::LPT;
     P.TB = TBL; P.TBP = TBL;
-    if ((P.in_split_len && (P.mode != CM_INV || P.in_split_len % G::RLAST)) || (P.out_split_len && (P.mode != CM_FWD || P.out_split_len % G::RLAST)))
-        throw Error("split row blocks are supported for forward-only outputs / inverse-only inputs, in multiples of the last radix");
     // side buffer (8 bytes per lane and padded position): next tile's input rows / this tile's real spectrum
     const size_t side_bytes = G::NST > 1 ? (size_t)(C::Ln + C::Ln / G::RLAST) * C::NLC * 8 : 0;
-    static const char* env_ns = getenv("HIPGP_NO_STAGE");
-    const bool use_side = G::NST > 1 && !env_ns;
-    P.spec_stage = (use_side && P.mode == CM_FUSED && P.spec_kind == SPEC_REAL) ? 1 : 0;
-    P.in_stage = (use_side && P.mode != CM_INV && (size_t)P.n_in * C::NLC * 16 <= side_bytes) ? 1 : 0;
+    P.spec_stage = (G::NST > 1 && P.mode == CM_FUSED && P.spec_kind == SPEC_REAL) ? 1 : 0;
+    P.in_stage = (G::NST > 1 && P.mode != CM_INV && (size_t)P.n_in * C::NLC * 16 <= side_bytes) ? 1 : 0;
     const size_t smem = G::smem_bytes() + ((P.spec_stage || P.in_stage) ? side_bytes : 0);
     P.nx = (int)((P.inner + TBL - 1) / TBL); P.ny = (int)n_outer; P.nz = (int)B;
     // tile order: lines fastest keeps neighbouring CTAs on neighbouring 32/64-byte row segments (shared DRAM bursts); but a
@@ -148,20 +141,12 @@ template <class T, int LEN, int R0, int R1, int R2> struct ColsBlkLaunch<T, LEN,
         // (measured, profiles/README.md r2c: a gain where the twiddle tables fit next to the tile -- fp32 --, a loss otherwise)
         if constexpr (!Cfg::ok) { (void)pl; (void)P; (void)n_outer; (void)B; (void)st; return false; }
         else {
-            static const char* env_blk = getenv("HIPGP_COLS_BLK");
-            if (env_blk && env_blk[0] == '0') return false;
-            static const char* env_tws = getenv("HIPGP_BLK_NEEDS_TWS");      // A/B: restrict to lists whose twiddle tables fit in shared memory
-            if (!Cfg::tw_smem && env_tws && env_tws[0] == '1') return false;
             if ((long)((P.inner + C::NLC * C::LPT - 1) / (C::NLC * C::LPT)) * n_outer * B >= (1L << 31)) return false;
             using G = typename Cfg::G;
             constexpr int TBL = C::NLC * C::LPT;
             P.TB = TBL; P.TBP = TBL;
-            if ((P.in_split_len && (P.mode != CM_INV || P.in_split_len % G::RLAST)) || (P.out_split_len && (P.mode != CM_FWD || P.out_split_len % G::RLAST)))
-                throw Error("split row blocks are supported for forward-only outputs / inverse-only inputs, in multiples of the last radix");
-            static const char* env_ns = getenv("HIPGP_NO_STAGE");
-            const bool use_side = !env_ns;
-            P.spec_stage = (use_side && P.mode == CM_FUSED && P.spec_kind == SPEC_REAL) ? 1 : 0;
-            P.in_stage = (use_side && P.mode != CM_INV && (size_t)P.n_in * C::NLC * 16 <= Cfg::side_bytes) ? 1 : 0;
+            P.spec_stage = (P.mode == CM_FUSED && P.spec_kind == SPEC_REAL) ? 1 : 0;
+            P.in_stage = (P.mode != CM_INV && (size_t)P.n_in * C::NLC * 16 <= Cfg::side_bytes) ? 1 : 0;
             const size_t smem = Cfg::smem_bytes;
             P.nx = (int)((P.inner + TBL - 1) / TBL); P.ny = (int)n_outer; P.nz = (int)B;
             {
@@ -173,24 +158,21 @@ template <class T, int LEN, int R0, int R1, int R2> struct ColsBlkLaunch<T, LEN,
             // the real spectrum tile as one padded box.  Anything else keeps the cp.async staging.
             ColsTmaMaps maps{};
             P.tma_in = P.tma_spec = 0;
-            static const char* env_nt = getenv("HIPGP_NO_TMA_COLS");
-            if (!env_nt) {
-                constexpr int HALF = C::Ln / 2;
-                const int nbox = (HALF + 255) / 256;
-                if (P.in_stage && P.n_in <= HALF && P.in_ostride == 0 && n_outer == 1 && HALF % nbox == 0 && is_pow2(R0)) {
-                    const unsigned long long dim[3] = {(unsigned long long)(2 * P.pitch), (unsigned long long)P.n_in, (unsigned long long)B};
-                    const unsigned long long bstr = (unsigned long long)(P.in_bstride ? P.in_bstride : (long)P.n_in * P.pitch);
-                    const unsigned long long str[2] = {(unsigned long long)P.pitch * sizeof(cplx<T>), bstr * sizeof(cplx<T>)};
-                    const unsigned box[3] = {(unsigned)(2 * TBL), (unsigned)(HALF / nbox), 1u};
-                    if (encode_map3(&maps.in, P.in, (int)sizeof(T), dim, str, box)) { P.tma_in = 1; P.tma_in_rows = HALF / nbox; P.tma_in_nbox = nbox; }
-                }
-                if (P.spec_stage && C::Ln / R2 <= 256 && (TBL * sizeof(T)) % 16 == 0) {
-                    const long sp = P.spec_pitch ? P.spec_pitch : P.pitch;
-                    const unsigned long long dim[3] = {(unsigned long long)sp, (unsigned long long)R2, (unsigned long long)(C::Ln / R2)};
-                    const unsigned long long str[2] = {(unsigned long long)sp * sizeof(T), (unsigned long long)sp * R2 * sizeof(T)};
-                    const unsigned box[3] = {(unsigned)TBL, (unsigned)(R2 + 1), (unsigned)(C::Ln / R2)};
-                    if (encode_map3(&maps.spec, P.spec, (int)sizeof(T), dim, str, box)) P.tma_spec = 1;
-                }
+            constexpr int HALF = C::Ln / 2;
+            const int nbox = (HALF + 255) / 256;
+            if (P.in_stage && P.n_in <= HALF && P.in_ostride == 0 && n_outer == 1 && HALF % nbox == 0 && is_pow2(R0)) {
+                const unsigned long long dim[3] = {(unsigned long long)(2 * P.pitch), (unsigned long long)P.n_in, (unsigned long long)B};
+                const unsigned long long bstr = (unsigned long long)(P.in_bstride ? P.in_bstride : (long)P.n_in * P.pitch);
+                const unsigned long long str[2] = {(unsigned long long)P.pitch * sizeof(cplx<T>), bstr * sizeof(cplx<T>)};
+                const unsigned box[3] = {(unsigned)(2 * TBL), (unsigned)(HALF / nbox), 1u};
+                if (encode_map3(&maps.in, P.in, (int)sizeof(T), dim, str, box)) { P.tma_in = 1; P.tma_in_rows = HALF / nbox; P.tma_in_nbox = nbox; }
+            }
+            if (P.spec_stage && C::Ln / R2 <= 256 && (TBL * sizeof(T)) % 16 == 0) {
+                const long sp = P.spec_pitch ? P.spec_pitch : P.pitch;
+                const unsigned long long dim[3] = {(unsigned long long)sp, (unsigned long long)R2, (unsigned long long)(C::Ln / R2)};
+                const unsigned long long str[2] = {(unsigned long long)sp * sizeof(T), (unsigned long long)sp * R2 * sizeof(T)};
+                const unsigned box[3] = {(unsigned)TBL, (unsigned)(R2 + 1), (unsigned)(C::Ln / R2)};
+                if (encode_map3(&maps.spec, P.spec, (int)sizeof(T), dim, str, box)) P.tma_spec = 1;
             }
             auto k = cols_blk_kernel<T, C::NLC, C::NTC, C::MINBC, R0, R1, R2>;
             if (smem > 40 * 1024) HIPGP_SET_MAX_SMEM(k, smem);
@@ -212,8 +194,7 @@ static bool cols_lane_aligned(const ColsParams<T>& P) {
     constexpr long A = 16 / (long)sizeof(cplx<T>);          // complex elements per 16 bytes (2 for fp32, 1 for fp64)
     auto al = [&](long v) { return v % A == 0; };
     return ((uintptr_t)P.in % 16 == 0) && ((uintptr_t)P.out % 16 == 0) && ((uintptr_t)P.spec % 16 == 0) && al(P.pitch) && al(P.in_ostride) &&
-           al(P.in_bstride) && al(P.out_ostride) && al(P.out_bstride) && al(P.in_split_stride) && al(P.out_split_stride) &&
-           al(P.spec_pitch);
+           al(P.in_bstride) && al(P.out_ostride) && al(P.out_bstride) && al(P.spec_pitch);
 }
 
 template <class T, int LEN> struct FastList;

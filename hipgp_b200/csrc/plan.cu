@@ -6,7 +6,6 @@
 
 namespace hipgp {
 thread_local std::string g_err;
-bool g_no_fast = false;
 }
 
 namespace hipgp {
@@ -31,7 +30,6 @@ template <class T> static bool aligned2(const void* p) { return ((uintptr_t)p % 
 
 template <class T>
 static bool launch_rows_fast(hipgp_plan* pl, bool inverse, RowsParams<T>& P, cudaStream_t st) {
-    if (g_no_fast) return false;
     switch (P.H) {
 #define X(LEN, ...) case LEN: launch_rows_fast_len<T, LEN>(pl, inverse, P, st); return true;
         HIPGP_FAST_LIST(X)
@@ -46,7 +44,7 @@ static bool launch_rows_fast(hipgp_plan* pl, bool inverse, RowsParams<T>& P, cud
 template <class T>
 static bool geom_allows_fast(const Geom<T>& g) {
     if (sizeof(T) == 8) return true;
-    if (g_no_fast || fast_radices(g.H).empty()) return false;
+    if (fast_radices(g.H).empty()) return false;
     for (int d = 0; d + 1 < g.D; ++d) if (fast_radices(g.L[d]).empty()) return false;
     return true;
 }
@@ -80,7 +78,6 @@ static void launch_rows(hipgp_plan* pl, bool inverse, RowsParams<T>& P, cudaStre
 
 template <class T>
 static bool launch_cols_fast(hipgp_plan* pl, ColsParams<T>& P, long n_outer, long B, cudaStream_t st) {
-    if (g_no_fast) return false;
     switch (P.f.Ln) {
 #define X(LEN, ...) case LEN: return launch_cols_fast_len<T, LEN>(pl, P, n_outer, B, st);
         HIPGP_FAST_LIST(X)
@@ -133,7 +130,7 @@ static void ws_elems(int D, const int* L, long P, const int* n_in, const int* n_
 
 // The pruned D-dimensional circular convolution:  out = crop_{n_out} IFFT( spec * FFT pad_{n_in} in ).
 template <class T>
-static void run_pipeline_group(hipgp_plan* pl, Geom<T>& g, const int* n_in, const int* n_out, const void* spec, int spec_kind,
+static void run_pipeline(hipgp_plan* pl, Geom<T>& g, const int* n_in, const int* n_out, const void* spec, int spec_kind,
                          long B, const RowsFusion& ff, const RowsFusion& fi, const PcgDev& st, bool gated, cudaStream_t s) {
     const int D = g.D;
     long w1, w2;
@@ -192,54 +189,6 @@ static void run_pipeline_group(hipgp_plan* pl, Geom<T>& g, const int* n_in, cons
     R.total_rows = B * rows_out; R.nrows = (int)rows_out; R.n_real = n_out[D - 1];
     if (D == 1) { R.spec = spec; R.spec_kind = spec_kind; }
     launch_rows<T>(pl, true, R, s, fast);
-}
-
-
-// Right-hand sides per pass group (an experiment kept behind HIPGP_L2_GROUP_MB, default off).  Idea: 3-D pipelines make five
-// passes over two workspaces; if the workspaces of a GROUP of right-hand sides fit the 126 MB L2 together, every pass after
-// the first finds its input there instead of in HBM.  Measured on a B200 (profiles/README.md r2f, cfg4 B = 200 K matvec):
-// 7.21 ms ungrouped, 8.7 / 9.5 / 11.1 ms with 120 / 80 / 40 MB groups -- the small launches lose more than the L2 hits
-// return (the passes are issue / latency bound, not HBM bound), as at cfg2 in round 1.  So whole batches by default.
-template <class T>
-static long pass_group(hipgp_plan* pl, Geom<T>& g, const int* n_in, const int* n_out, long B) {
-    static const char* env = getenv("HIPGP_L2_GROUP_MB");
-    const double budget_mb = env ? atof(env) : 0.0;
-    if (budget_mb <= 0 || B <= 1) return B;
-    long w1, w2;
-    ws_elems(g.D, g.L, g.P, n_in, n_out, 1, &w1, &w2);
-    long vin = 1, vout = 1;
-    for (int d = 0; d < g.D; ++d) { vin *= n_in[d]; vout *= n_out[d]; }
-    const double per_rhs = (double)sizeof(cplx<T>) * (double)(w1 + w2) + (double)sizeof(T) * (double)(vin + vout);
-    long grp = (long)(budget_mb * 1048576.0 / per_rhs);
-    (void)pl;
-    return std::max<long>(1, std::min<long>(B, grp));
-}
-
-template <class T>
-static void run_pipeline(hipgp_plan* pl, Geom<T>& g, const int* n_in, const int* n_out, const void* spec, int spec_kind,
-                         long B, const RowsFusion& ff, const RowsFusion& fi, const PcgDev& st, bool gated, cudaStream_t s) {
-    const long grp = pass_group<T>(pl, g, n_in, n_out, B);
-    if (grp >= B) { run_pipeline_group<T>(pl, g, n_in, n_out, spec, spec_kind, B, ff, fi, st, gated, s); return; }
-    long vin = 1, vout = 1, rows_in = 1, rows_out = 1;
-    for (int d = 0; d < g.D; ++d) { vin *= n_in[d]; vout *= n_out[d]; }
-    for (int d = 0; d + 1 < g.D; ++d) { rows_in *= n_in[d]; rows_out *= n_out[d]; }
-    auto shift = [](const void* p, long elems) -> const void* { return p ? (const void*)((const T*)p + elems) : nullptr; };
-    for (long b0 = 0; b0 < B; b0 += grp) {
-        const long nb = std::min(grp, B - b0);
-        RowsFusion f2 = ff, i2 = fi;
-        // forward-side vectors have the input extents, inverse-side vectors the output extents (PCG: both are M)
-        f2.in = shift(ff.in, b0 * vin); f2.v0 = (void*)shift(ff.v0, b0 * vin); f2.v1 = (void*)shift(ff.v1, b0 * vin); f2.v2 = shift(ff.v2, b0 * vin);
-        i2.out = (void*)shift(fi.out, b0 * vout); i2.v0 = (void*)shift(fi.v0, b0 * vout);
-        PcgDev s2 = st;
-        if (st.zr) {          // per-right-hand-side scalars / counters of this group; the stop test still spans all B
-            s2.zr = st.zr + b0; s2.zr_prev = st.zr_prev + b0; s2.pAp = st.pAp + b0; s2.rr = st.rr + b0;
-            s2.rr_all = st.rr_all ? st.rr_all : st.rr;
-            s2.row_cnt = st.row_cnt + b0;
-            // partial sums: one slot per global row of the launch (forward launches count input rows, inverse ones output rows)
-            s2.partial = st.partial + b0 * std::max(rows_in, rows_out);
-        }
-        run_pipeline_group<T>(pl, g, n_in, n_out, spec, spec_kind, nb, f2, i2, s2, gated, s);
-    }
 }
 
 // forward-only transform of a real (L_0..L_{D-1}) fp64 array into W1 (raw spectrum, pipeline layout)
@@ -309,7 +258,6 @@ static void dct_all_axes(hipgp_plan* pl, const double* in, double* out, double* 
     const int D = pl->D;
     double* bufs[2] = {out, tmp};
     int which = (D % 2 == 1) ? 0 : 1;   // so that the last axis writes `out`
-    static const char* env_old = getenv("HIPGP_DCT_DENSE");       // A/B switch: the round-1 one-output-per-thread kernel
     for (int d = 0; d < D; ++d) {
         const int md = pl->m[d];
         long inner = 1, outer = 1;
@@ -319,15 +267,7 @@ static void dct_all_axes(hipgp_plan* pl, const double* in, double* out, double* 
         const int Nn = md > 1 ? 2 * (md - 1) : 1;
         double* dst = bufs[which];
         const double scale = normalise ? 1.0 / (double)Nn : 1.0;
-        if (env_old) {
-            int bx = 64;
-            while (bx > 1 && bx / 2 >= inner) bx >>= 1;
-            dim3 block(bx, 256 / bx);
-            const int nx = (int)((inner + bx - 1) / bx);
-            dim3 grid((unsigned)((long)nx * outer), (unsigned)((md + block.y - 1) / block.y), 1);
-            auto k = dct1_axis_kernel;
-            HIPGP_LAUNCH(k, grid, block, 0, s, src, dst, tab, md, inner, scale, nx);
-        } else if (inner == 1) {
+        if (inner == 1) {
             dim3 grid((unsigned)((md + 63) / 64), (unsigned)((outer + 127) / 128), 1);      // 128 x 64 output tile per block
             const double* cw = md > 2 ? axis_cosmat(pl, d, s) : nullptr;
             if (cw) {      // reflection symmetry folded in: two half-size products, one per output parity (grid.z)
@@ -442,9 +382,8 @@ static void ensure_wide(hipgp_plan* pl, cudaStream_t s) {
     ensure_geoms<T>(pl, true);
     // Where every axis of the wide embedding is at least 2N - 1 long (config 2: 4096 >= 3995, the length the cost model picks
     // anyway) the taps are extended symmetrically and the spectrum of C^(1/2) is REAL: R^T and R then take the same staged
-    // real-spectrum column pass as K instead of reading a complex spectrum from global memory (HIPGP_WIDE_COMPLEX=1: A/B switch).
-    static const char* env_c = getenv("HIPGP_WIDE_COMPLEX");
-    bool real_ok = !env_c;
+    // real-spectrum column pass as K instead of reading a complex spectrum from global memory.
+    bool real_ok = true;
     for (int d = 0; d < pl->D; ++d) if (pl->Lw[d] < 2 * pl->N[d] - 1) real_ok = false;
     pl->wide_real = real_ok;
     dct_all_axes(pl, pl->Dsqrt.as<double>(), pl->colS.as<double>(), pl->tmpB.as<double>(), true, s);
@@ -669,14 +608,10 @@ int hipgp_plan_create(int ndim, const int64_t* m, int dtype, int device, hipgp_p
     }
     if (D == 0) { D = 1; pl->m[0] = 1; pl->N[0] = 1; }
     pl->D = D;
-    const char* nf = getenv("HIPGP_NO_FAST");
-    g_no_fast = nf && nf[0] == '1';
-    const char* env = getenv("HIPGP_POW2_ONLY");
-    const bool pow2 = env && env[0] == '1';
     for (int d = 0; d < D; ++d) {
         const bool row = (d == D - 1);
-        pl->Ln[d] = choose_length(2L * pl->m[d] - 1, row, pow2);
-        pl->Lw[d] = choose_length((long)pl->N[d] + pl->m[d] - 1, row, pow2);
+        pl->Ln[d] = choose_length(2L * pl->m[d] - 1, row);
+        pl->Lw[d] = choose_length((long)pl->N[d] + pl->m[d] - 1, row);
     }
     *out = pl;
     API_END
@@ -688,7 +623,7 @@ int hipgp_plan_destroy(hipgp_plan* pl) {
     size_t* t = &pl->dev_bytes;
     pl->gn32.release(t); pl->gw32.release(t); pl->gn64.release(t); pl->gw64.release(t);
     for (DevBuf* b : {&pl->specK, &pl->specCinv, &pl->specW, &pl->Dm, &pl->Dinv, &pl->Dsqrt, &pl->colK, &pl->colG, &pl->colS,
-                      &pl->tmpA, &pl->tmpB, &pl->costab, &pl->counts, &pl->W1, &pl->W2, &pl->vr, &pl->vp, &pl->vz, &pl->vAp,
+                      &pl->tmpA, &pl->tmpB, &pl->counts, &pl->W1, &pl->W2, &pl->vr, &pl->vp, &pl->vz, &pl->vAp,
                       &pl->partial, &pl->scal, &pl->cnt, &pl->flags, &pl->stage_in, &pl->stage_out, &pl->corrU, &pl->corrV, &pl->corrS,
                       &pl->corrLag, &pl->gradA, &pl->slabSpecK, &pl->slabSpecCinv, &pl->slabR1, &pl->slabR2, &pl->slot_in[0], &pl->slot_in[1], &pl->slot_out[0], &pl->slot_out[1], &pl->costabs[0], &pl->costabs[1], &pl->costabs[2], &pl->cosmats[0], &pl->cosmats[1], &pl->cosmats[2]})
         b->release(t);

@@ -62,8 +62,6 @@ struct DevBuf {
 #endif
 #define HIPGP_FAST_LIST(X) HIPGP_FAST_LIST_G0(X) HIPGP_FAST_LIST_G1(X) HIPGP_FAST_LIST_G2(X) HIPGP_FAST_LIST_G3(X) HIPGP_FAST_LIST_G4(X)
 
-extern bool g_no_fast;
-
 inline std::vector<int> fast_radices(int Ln) {
     switch (Ln) {
 #define X(LEN, ...) case LEN: return std::vector<int>{__VA_ARGS__};
@@ -102,12 +100,12 @@ inline bool is_smooth(long n) {
 }
 
 // smallest-cost 2^a 3^b 5^c length >= n (even when `even`), searched in [n, 2n]
-inline int choose_length(long n, bool even, bool pow2_only) {
+inline int choose_length(long n, bool even) {
     if (n < 2) n = 2;
     long best = -1; double bc = 0;
     for (long L = n; L <= 2 * n + 2; ++L) {
         if (even && (L & 1)) continue;
-        if (pow2_only ? ((L & (L - 1)) != 0) : !is_smooth(L)) continue;
+        if (!is_smooth(L)) continue;
         const double c = even ? 2.0 * fft_cost((int)(L / 2)) : fft_cost((int)L);
         if (best < 0 || c < bc) { best = L; bc = c; }
     }
@@ -282,11 +280,11 @@ struct hipgp_plan {
     Geom<float> gn32, gw32;    // narrow (K, Cinv) / wide (RT, R) geometries in the plan dtype
     Geom<double> gn64, gw64;   // fp64 geometries (set-up always runs in fp64; also the fp64 plan's own)
     DevBuf specK, specCinv, specW;         // stored spectra (plan dtype; specW complex)
-    DevBuf Dm, Dinv, Dsqrt, colK, colG, colS, tmpA, tmpB, costab, counts;   // fp64 set-up arrays (M each)
+    DevBuf Dm, Dinv, Dsqrt, colK, colG, colS, tmpA, tmpB, counts;   // fp64 set-up arrays (M each)
     DevBuf W1, W2;                         // frequency-domain workspace
     DevBuf vr, vp, vz, vAp, partial, scal, cnt, flags;   // PCG state
     DevBuf stage_in, stage_out;            // device staging for the *_host entry points
-    DevBuf slabSpecK, slabSpecCinv;        // this rank's bins of the spectra, [L0][L1][Pq] (slab decomposition v2)
+    DevBuf slabSpecK, slabSpecCinv;        // this rank's bins of the spectra, [L0][L1][Pq] (slab decomposition)
     bool have_slabK = false, have_slabCinv = false;
     DevBuf costabs[3], cosmats[3];                     // DCT-I cosine tables per active axis (built once per plan)
     DevBuf gradA;                          // R^T column gradient (corr_api.inl): one M-sized fp64 work array

@@ -15,33 +15,9 @@ namespace hipgp {
 
 // out[o][k][i] = sum_j w_j in[o][j][i] cos(pi j k / (m-1)),  w_0 = w_{m-1} = 1, else 2.   (DCT-I, unnormalised;
 // applying it twice multiplies by N = 2(m-1)).  costab[t] = cos(pi t / (m-1)), t in [0, 2(m-1)).
-// block (bx, 256/bx) with bx = min(64, inner); grid.x = ceil(inner/bx) * outer (outer folded into x: no 65535 limit),
-// grid.y = ceil(m / blockDim.y)
-__global__ void __launch_bounds__(256) dct1_axis_kernel(const double* __restrict__ in, double* __restrict__ out,
-                                                        const double* __restrict__ costab, int m, long inner, double scale, int nx) {
-    const long ob = blockIdx.x / nx, xb = blockIdx.x - ob * nx;
-    const long i = xb * blockDim.x + threadIdx.x;
-    const int k = blockIdx.y * blockDim.y + threadIdx.y;
-    if (i >= inner || k >= m) return;
-    const size_t o = (size_t)ob * m * inner;
-    const int N = 2 * (m - 1);
-    double acc = 0.0;
-    if (m == 1) {
-        acc = in[o + i];
-    } else {
-        int t = 0;   // (j*k) mod N, updated incrementally
-        for (int j = 0; j < m; ++j) {
-            const double w = (j == 0 || j == m - 1) ? 1.0 : 2.0;
-            acc += w * in[o + (size_t)j * inner + i] * costab[t];
-            t += k; if (t >= N) t -= N;
-        }
-    }
-    out[o + (size_t)k * inner + i] = acc * scale;
-}
-
-// The same DCT-I as a TILED fp64 contraction (round 2: the dense transform above is the one genuine matrix product of the
-// path -- (m x m cosine matrix) x (m x inner) per outer index -- and at config 2 the one-output-per-thread kernel above spent
-// 1.13 ms per launch, 8 launches per spectrum set-up).  64 x 64 output tile per CTA, 16-deep k tiles in shared memory,
+// It is the one genuine matrix product of the path -- (m x m cosine matrix) x (m x inner) per outer index -- so it runs as a
+// TILED fp64 contraction (a one-output-per-thread kernel spent 1.13 ms per launch at config 2, 8 launches per spectrum
+// set-up).  64 x 64 output tile per CTA, 16-deep k tiles in shared memory,
 // 16 x 16 threads with 4 x 4 fp64 accumulators each; the cosine operand is generated from the length-N table (index
 // (j k) mod N) while its tile is staged, so no m x m matrix is stored (axes longer than 2048 points; shorter axes take
 // dct1_sym_kernel below).

@@ -1,15 +1,11 @@
 """Slab-decomposed structured K_uu for grids sharded over several GPUs (SURVEY.md 8e, BASELINE config 5).
 
 Axis 0 of a 3-D grid is split contiguously over the ranks.  A matvec is three local stages with two all-to-all
-transposes between them (NCCL via torch.distributed).  Two layouts of what travels:
-
-  layout="bins" (default, round 2): the UN-PADDED output of the row pass, split along the bins of the last axis; after the
-      exchange a rank owns every (i0, i1) for its bins and runs the three ordinary column passes locally.  Half the bytes on
-      the wire of the first version.
-      exchange="peer" (default): no collective library on the data path -- the packing kernels store the blocks straight into
-      the peers' receive buffers over NVLink; exchange="nccl": all_to_all_single, optionally cut into `chunks` overlapped pieces.
-  layout="axis1" (round 1): the zero-padded axis-1 transform, split along axis-1 positions; the column passes next to each
-      transpose write / read the exchange buffer in its packed layout.
+transposes between them.  What travels is the UN-PADDED output of the row pass, split along the bins of the last axis; after
+the exchange a rank owns every (i0, i1) for its bins and runs the three ordinary column passes locally.
+  exchange="peer" (default): no collective library on the data path -- the packing kernels store the blocks straight into
+      the peers' receive buffers over NVLink; exchange="nccl": all_to_all_single (torch.distributed), cut into `chunks`
+      overlapped pieces (default 2).
 
 PCG on slab vectors is the reference's conj_grad2 with the dot products summed over ranks (one small all-reduce per dot).
 
@@ -17,7 +13,6 @@ PCG on slab vectors is the reference's conj_grad2 with the dot products summed o
 `emulate=True` runs all ranks inside one process on one GPU (lists of slabs in, lists out) -- used by the tests.
 """
 import ctypes as C
-import os
 
 import torch
 import torch.distributed as dist
@@ -28,19 +23,16 @@ from .cg import conj_grad2
 
 
 class SlabToeplitz:
-    def __init__(self, dims, column, dtype, device, rank=None, nranks=None, emulate_ranks=None, layout=None, chunks=None, exchange=None):
+    def __init__(self, dims, column, dtype, device, rank=None, nranks=None, emulate_ranks=None, chunks=None, exchange=None):
         assert len(dims) == 3, "slab decomposition is implemented for 3-D grids"
-        layout = layout or os.environ.get("HIPGP_SLAB_LAYOUT", "bins")
-        assert layout in ("bins", "axis1")
-        self.layout = layout
-        # bins layout: cut the exchange into `chunks` independent all-to-alls so that the column passes of one chunk run
-        # while its neighbours are on the wire (NCCL's stream next to the compute stream)
         # how the blocks travel: "peer" = the packing kernels store straight into the peers' receive buffers over NVLink (CUDA
         # inter-process handles, two small all-reduces per matvec as barriers); "nccl" = all_to_all_single between the stages
-        exchange = exchange or os.environ.get("HIPGP_SLAB_EXCHANGE", "peer" if layout == "bins" else "nccl")
-        assert exchange in ("peer", "nccl") and (exchange == "nccl" or layout == "bins")
+        exchange = exchange or "peer"
+        assert exchange in ("peer", "nccl")
         self.exchange = exchange
-        self.chunks = int(chunks or os.environ.get("HIPGP_SLAB_CHUNKS", "1" if exchange == "peer" else "2")) if layout == "bins" else 1
+        # cut the exchange into `chunks` independent all-to-alls so that the column passes of one chunk run while its
+        # neighbours are on the wire (NCCL's stream next to the compute stream)
+        self.chunks = int(chunks or (1 if exchange == "peer" else 2))
         self.dims = tuple(int(d) for d in dims)
         self.emulated = emulate_ranks is not None
         if self.emulated:
@@ -58,14 +50,18 @@ class SlabToeplitz:
             self.plans.append(p)
         p0 = self.plans[0]
         a, b = C.c_int64(), C.c_int64()
-        sizes = p0.lib.hipgp_slab2_sizes if layout == "bins" else p0.lib.hipgp_slab_sizes
-        L.check(p0.lib, sizes(p0._h, C.byref(a), C.byref(b)))
+        L.check(p0.lib, p0.lib.hipgp_slab2_sizes(p0._h, C.byref(a), C.byref(b)))
         self.slab_elems, self.exch_elems = a.value, b.value
         self.dtype, self.device = dtype, p0.device
         self.cdtype = torch.complex64 if dtype == torch.float32 else torch.complex128
         self.slab_shape = (self.dims[0] // self.nranks, self.dims[1], self.dims[2])
         if self.exchange == "peer":
             self._connect_peers()
+
+    @property
+    def layout(self):
+        """what travels between the stages: the row pass's un-padded output split along the last-axis bins"""
+        return "bins"
 
     def _connect_peers(self):
         """every rank allocates its two receive buffers and maps everybody else's"""
@@ -117,21 +113,16 @@ class SlabToeplitz:
     def _s1(self, p, v):
         send = torch.empty(self.exch_elems, dtype=self.cdtype, device=self.device)
         v = v.reshape(-1).to(self.dtype).contiguous()
-        f = p.lib.hipgp_slab2_stage_a if self.layout == "bins" else p.lib.hipgp_slab_stage1
-        L.check(p.lib, f(p._h, C.c_void_p(v.data_ptr()), C.c_void_p(send.data_ptr()), _stream_ptr(self.device)))
+        L.check(p.lib, p.lib.hipgp_slab2_stage_a(p._h, C.c_void_p(v.data_ptr()), C.c_void_p(send.data_ptr()), _stream_ptr(self.device)))
         return send
 
     def _s2(self, p, mode, buf, chunk=-1):
-        if self.layout == "bins":
-            L.check(p.lib, p.lib.hipgp_slab2_stage_b_chunk(p._h, mode, C.c_void_p(buf.data_ptr()), chunk, _stream_ptr(self.device)))
-        else:
-            L.check(p.lib, p.lib.hipgp_slab_stage2(p._h, mode, C.c_void_p(buf.data_ptr()), _stream_ptr(self.device)))
+        L.check(p.lib, p.lib.hipgp_slab2_stage_b_chunk(p._h, mode, C.c_void_p(buf.data_ptr()), chunk, _stream_ptr(self.device)))
         return buf
 
     def _s3(self, p, buf):
         out = torch.empty(self.slab_elems, dtype=self.dtype, device=self.device)
-        f = p.lib.hipgp_slab2_stage_c if self.layout == "bins" else p.lib.hipgp_slab_stage3
-        L.check(p.lib, f(p._h, C.c_void_p(buf.data_ptr()), C.c_void_p(out.data_ptr()), _stream_ptr(self.device)))
+        L.check(p.lib, p.lib.hipgp_slab2_stage_c(p._h, C.c_void_p(buf.data_ptr()), C.c_void_p(out.data_ptr()), _stream_ptr(self.device)))
         return out
 
     def _exchange(self, bufs):
@@ -149,7 +140,7 @@ class SlabToeplitz:
         return [recv]
 
     def _matvec_overlapped(self, mode, v):
-        """bins layout, several chunks, one rank per process: chunk c's column passes run while chunk c+1 arrives and chunk
+        """several chunks, one rank per process: chunk c's column passes run while chunk c+1 arrives and chunk
         c-1 already travels back (the collectives sit on NCCL's stream, ordered among themselves as issued)."""
         p = self.plans[0]
         per = self.exch_elems // self.chunks

@@ -186,22 +186,13 @@ int hipgp_rt_column_grad(hipgp_plan* plan, const void* vec_dev, const void* grad
                          void* stream);
 
 /* ---- slab-decomposed 3-D grids (axis 0 split over `nranks` GPUs; K and C^-1 matvecs; one right-hand side).
- * The reference has no multi-GPU path; this is the grid-sharded route of SURVEY.md 8e.  A matvec is
- *   stage1(in_slab -> send) ; all-to-all(send -> buf) ; stage2(mode, buf in place) ; all-to-all(buf -> recv) ;
- *   stage3(recv -> out_slab)
- * with the two all-to-alls issued by the caller (NCCL through torch.distributed); the passes next to them read / write
- * the exchange buffers in their packed layout directly, so there is no separate pack / unpack kernel.
- * Buffers: slab = (n0/nranks, m1, m2) reals; exchange = `exchange_complex` complex numbers. */
-int hipgp_plan_set_slab(hipgp_plan* plan, int rank, int nranks);
-int hipgp_slab_sizes(const hipgp_plan* plan, int64_t* slab_reals, int64_t* exchange_complex);
-int hipgp_slab_stage1(hipgp_plan* plan, const void* in_slab_dev, void* send_buf_dev, void* stream);
-int hipgp_slab_stage2(hipgp_plan* plan, int mode, void* buf_dev, void* stream);
-int hipgp_slab_stage3(hipgp_plan* plan, const void* recv_buf_dev, void* out_slab_dev, void* stream);
-/* version 2 of the same decomposition: what travels is the UN-PADDED output of the row pass, split along the bins of the last
- * axis (half the bytes of version 1, whose exchange carried the zero-padded axis-1 transform); after the exchange a rank owns
- * all (i0, i1) for its bins and runs the three ordinary column passes locally:
+ * The reference has no multi-GPU path; this is the grid-sharded route of SURVEY.md 8e.  What travels is the UN-PADDED output
+ * of the row pass, split along the bins of the last axis; after the exchange a rank owns all (i0, i1) for its bins and runs
+ * the three ordinary column passes locally:
  *   stage_a(in_slab -> send) ; all-to-all(send -> buf) ; stage_b(mode, buf in place) ; all-to-all(buf -> recv) ; stage_c(recv -> out_slab)
- * exchange buffers hold `exchange_complex` complex numbers = nranks equal blocks. */
+ * with the two all-to-alls issued by the caller (NCCL through torch.distributed), or the peer-memory exchange below.
+ * Buffers: slab = (n0/nranks, m1, m2) reals; exchange = `exchange_complex` complex numbers = nranks equal blocks. */
+int hipgp_plan_set_slab(hipgp_plan* plan, int rank, int nranks);
 int hipgp_slab2_sizes(const hipgp_plan* plan, int64_t* slab_reals, int64_t* exchange_complex);
 int hipgp_slab2_stage_a(hipgp_plan* plan, const void* in_slab_dev, void* send_buf_dev, void* stream);
 int hipgp_slab2_stage_b(hipgp_plan* plan, int mode, void* buf_dev, void* stream);

@@ -1,5 +1,6 @@
-"""Run under torchrun (N >= 2): slab-decomposed K matvec and PCG over NCCL all-to-all vs the undecomposed plan on rank 0.
-usage: check_slab.py [m0 m1 m2] [bench]"""
+"""Run under torchrun (N >= 2): slab-decomposed K matvec and PCG vs the undecomposed plan on rank 0.
+usage: check_slab.py [m0 m1 m2] [bench] [nccl]
+  nccl: exchange through NCCL all-to-alls (two overlapped chunks) instead of the peer-memory stores"""
 import os, sys, json
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch, torch.distributed as dist
@@ -11,14 +12,14 @@ torch.cuda.set_device(local); dev = torch.device("cuda", local)
 os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
 if world > 1:
     dist.init_process_group("nccl", device_id=dev)
-args = [a for a in sys.argv[1:] if a != "bench"]
+args = [a for a in sys.argv[1:] if a not in ("bench", "nccl")]
 dims = tuple(int(a) for a in args[:3]) if len(args) >= 3 else (64, 48, 40)
 bench = "bench" in sys.argv
 dtype = torch.float32 if bench else torch.float64
 xg = [torch.linspace(0, 1, m, dtype=dtype, device=dev) for m in dims]
 step = float(xg[0][1] - xg[0][0])
 col = hk.first_row(xg, hk.Matern(nu=2.5, dtype=dtype), (1.0, 2.5 * step), jitter=1e-3)
-slab = SlabToeplitz(dims, col, dtype, dev)
+slab = SlabToeplitz(dims, col, dtype, dev, exchange="nccl" if "nccl" in sys.argv else None)
 n0 = dims[0] // world
 gen = torch.Generator(device=dev); gen.manual_seed(42)
 v = torch.randn(1, int(np.prod(dims)), dtype=dtype, device=dev, generator=gen)      # same on every rank

@@ -15,16 +15,14 @@ def mkplan(dims, dt, col, slab=None, chunks=1):
     ncl = C.c_int64()
     assert lib.hipgp_plan_set_first_row(plan, ptr(col), 1e-6, C.byref(ncl), None) == 0, lib.hipgp_last_error()
     return plan
-def run(dims, nranks, dt, v2=False, chunks=1, peer=False):
+def run(dims, nranks, dt, chunks=1, peer=False):
     g = np.meshgrid(*[np.linspace(0, 1 + d, k) for d, k in enumerate(dims)], indexing="ij")
     r = np.sqrt(sum((x - x.flat[0]) ** 2 for x in g)); col = ((1 + np.sqrt(3) * r / 0.4) * np.exp(-np.sqrt(3) * r / 0.4)).reshape(-1); col[0] += 1e-2
     col = col.astype(dt)
     full = mkplan(dims, dt, col)
     plans = [mkplan(dims, dt, col, (rk, nranks), chunks) for rk in range(nranks)]
     a, b = C.c_int64(), C.c_int64()
-    st1, st2, st3, sz = ((lib.hipgp_slab2_stage_a, lib.hipgp_slab2_stage_b, lib.hipgp_slab2_stage_c, lib.hipgp_slab2_sizes) if v2 else
-                         (lib.hipgp_slab_stage1, lib.hipgp_slab_stage2, lib.hipgp_slab_stage3, lib.hipgp_slab_sizes))
-    assert sz(plans[0], C.byref(a), C.byref(b)) == 0, lib.hipgp_last_error(); slab_elems, exch = a.value, b.value
+    assert lib.hipgp_slab2_sizes(plans[0], C.byref(a), C.byref(b)) == 0, lib.hipgp_last_error(); slab_elems, exch = a.value, b.value
     rng = np.random.default_rng(0); M = int(np.prod(dims))
     v = rng.standard_normal((1, M)).astype(dt)
     n0 = dims[0] // nranks
@@ -54,20 +52,19 @@ def run(dims, nranks, dt, v2=False, chunks=1, peer=False):
             continue
         bufs = []
         for p, x in zip(plans, slabs):
-            send = np.zeros(exch, dtype=cdt); assert st1(p, ptr(x), ptr(send), None) == 0, lib.hipgp_last_error(); bufs.append(send)
+            send = np.zeros(exch, dtype=cdt); assert lib.hipgp_slab2_stage_a(p, ptr(x), ptr(send), None) == 0, lib.hipgp_last_error(); bufs.append(send)
         bufs = exchange(bufs)
-        for p, bb in zip(plans, bufs): assert st2(p, mode, ptr(bb), None) == 0, lib.hipgp_last_error()
+        for p, bb in zip(plans, bufs): assert lib.hipgp_slab2_stage_b(p, mode, ptr(bb), None) == 0, lib.hipgp_last_error()
         bufs = exchange(bufs)
         outs = []
         for p, bb in zip(plans, bufs):
-            o = np.zeros(slab_elems, dtype=dt); assert st3(p, ptr(bb), ptr(o), None) == 0, lib.hipgp_last_error(); outs.append(o)
+            o = np.zeros(slab_elems, dtype=dt); assert lib.hipgp_slab2_stage_c(p, ptr(bb), ptr(o), None) == 0, lib.hipgp_last_error(); outs.append(o)
         got = np.concatenate(outs).reshape(1, -1)
         e = np.linalg.norm(got - ref) / np.linalg.norm(ref)
-        print(dims, nranks, dt.__name__, "v2" if v2 else "v1", "chunks", chunks, "mode", mode, "err %.2e" % e); ok &= e < (1e-5 if dt == np.float32 else 1e-10)
+        print(dims, nranks, dt.__name__, "chunks", chunks, "mode", mode, "err %.2e" % e); ok &= e < (1e-5 if dt == np.float32 else 1e-10)
     return ok
 if __name__ == "__main__":
-    ok = run((16, 12, 20), 2, np.float64) & run((16, 12, 20), 4, np.float32)
-    ok &= run((16, 12, 20), 2, np.float64, True) & run((16, 12, 20), 4, np.float32, True) & run((12, 10, 14), 3, np.float64, True)
-    ok &= run((16, 12, 20), 4, np.float32, True, 1, True) & run((12, 10, 14), 3, np.float64, True, 2, True)
-    ok &= run((16, 12, 20), 2, np.float32, True, 2) & run((12, 10, 14), 3, np.float64, True, 3)
+    ok = run((16, 12, 20), 2, np.float64) & run((16, 12, 20), 4, np.float32) & run((12, 10, 14), 3, np.float64)
+    ok &= run((16, 12, 20), 4, np.float32, 1, True) & run((12, 10, 14), 3, np.float64, 2, True)
+    ok &= run((16, 12, 20), 2, np.float32, 2) & run((12, 10, 14), 3, np.float64, 3)
     sys.exit(0 if ok else 1)

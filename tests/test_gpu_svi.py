@@ -90,9 +90,9 @@ def test_begin_step_pcg_matches_fused_solve(golden_dir):
     assert relerr(torch.cat(xs), x_ref.cpu().numpy()) < 1e-12
 
 
-@pytest.mark.parametrize("layout,exchange", [("bins", "peer"), ("bins", "nccl"), ("axis1", "nccl")])
-@pytest.mark.parametrize("dname,nranks", [("f64", 2), ("f32", 4)])
-def test_slab_decomposed_matvec_emulated(dname, nranks, layout, exchange):
+@pytest.mark.parametrize("exchange", ["peer", "nccl"])
+@pytest.mark.parametrize("dname,nranks", [("f64", 2), ("f64", 4), ("f32", 2), ("f32", 4)])
+def test_slab_decomposed_matvec_emulated(dname, nranks, exchange):
     """Grid-sharded (slab) K and C^-1 matvecs: all ranks emulated on one GPU, the all-to-all done by tensor shuffling;
     must equal the undecomposed plan and the CPU oracle."""
     from hipgp_b200.slab import SlabToeplitz
@@ -103,7 +103,7 @@ def test_slab_decomposed_matvec_emulated(dname, nranks, layout, exchange):
     dims = (16, 12, 20)
     xg = [torch.linspace(0, 1 + d, m, dtype=dtype, device=DEV) for d, m in enumerate(dims)]
     col = hk.first_row(xg, hk.Matern(nu=1.5, dtype=dtype), (1.0, 0.4), jitter=1e-2)
-    slab = SlabToeplitz(dims, col, dtype, DEV, emulate_ranks=nranks, layout=layout, exchange=exchange)
+    slab = SlabToeplitz(dims, col, dtype, DEV, emulate_ranks=nranks, exchange=exchange)
     full = Plan(dims, dtype, DEV).set_first_row(col)
     torch.manual_seed(0)
     v = torch.randn(1, int(np.prod(dims)), dtype=dtype, device=DEV)
