@@ -43,6 +43,16 @@ template <class T> __device__ __forceinline__ T warp_sum(T v) {
     return v;
 }
 
+// The stopping rule all_b sqrt(r_b.r_b) < tol (cg.py:70), run by one thread once r.r of every right-hand side is in.
+__device__ __forceinline__ void pcg_stop_test(const PcgDev& st) {
+    bool all = true;
+    const volatile double* rr = st.rr_all ? st.rr_all : st.rr;
+    for (int i = 0; i < st.B; ++i) all = all && (sqrt(rr[i]) < st.tol);
+    st.flags[1] += 1;
+    st.flags[2] = 0;
+    if (all) st.flags[0] = 1;
+}
+
 // Deterministic finalisation: called by every thread of the CTA after it has written the per-row partials
 // of rows [g0, g1).  The CTA that completes a right-hand side sums that rhs's partials in a fixed order.
 __device__ __forceinline__ void pcg_finalize(const PcgDev& st, int kind, long g0, long g1, int nrows, int tid, int nthreads) {
@@ -84,13 +94,8 @@ __device__ __forceinline__ void pcg_finalize(const PcgDev& st, int kind, long g0
                     const unsigned nb = atomicAdd(st.rhs_cnt, 1u) + 1u;
                     if (nb == (unsigned)st.B) {
                         __threadfence();
-                        bool all = true;
-                        const volatile double* rr = st.rr_all ? st.rr_all : st.rr;
-                        for (int i = 0; i < st.B; ++i) all = all && (sqrt(rr[i]) < st.tol);
                         st.rhs_cnt[0] = 0;
-                        st.flags[1] += 1;
-                        st.flags[2] = 0;
-                        if (all) st.flags[0] = 1;
+                        pcg_stop_test(st);
                     }
                 }
             }

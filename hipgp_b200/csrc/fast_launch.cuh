@@ -51,6 +51,14 @@ static void launch_check(const char* what, int len, int nl, int nt, size_t smem,
                     ", shared " + std::to_string(smem) + " B, grid " + std::to_string(grid) + "): " + cudaGetErrorString(e));
 }
 
+// shared memory of a row-pass CTA: the tile, then the side buffer with the tile's real rows (row-major)
+template <class T, int... Rs>
+static size_t rows_fast_smem(long n_real) {
+    using C = FastCfg<T, Rs...>;
+    using G = TileGeo<T, C::NLR, Rs...>;
+    return G::smem_bytes() + sizeof(T) * (size_t)((n_real + 3) & ~3L) * (C::NLR * C::LPT);
+}
+
 template <class T, int... Rs>
 static void launch_rows_fast_t(hipgp_plan* pl, bool inverse, RowsParams<T>& P, cudaStream_t st) {
     using C = FastCfg<T, Rs...>;
@@ -63,9 +71,8 @@ static void launch_rows_fast_t(hipgp_plan* pl, bool inverse, RowsParams<T>& P, c
         const int want_q = NST > 1 ? (H - G::RLAST) / 4 : 0, want_p = NST > 1 ? G::RLAST / 2 + 1 : H / 2 + 1;
         if (P.nquad != want_q || P.npair0 != want_p) throw Error("internal: unexpected r2c pair structure for H = " + std::to_string(H));
     }
-    // the tile, then the side buffer: the tile's real rows, row-major
-    const size_t smem = G::smem_bytes() + sizeof(T) * (size_t)((P.n_real + 3) & ~3) * NROW;
-    if (smem > 227 * 1024) throw Error("row pass: rows too long for the shared-memory side buffer");
+    const size_t smem = rows_fast_smem<T, Rs...>(P.n_real);
+    if (smem > kRowsFastSmemMax) throw Error("row pass: rows too long for the shared-memory side buffer");
     // operands of a fused update land in the tile buffer: two row blocks must fit in it
     P.tma_op = (!inverse && 2 * sizeof(T) * (size_t)((P.n_real + 3) & ~3) * NROW <= G::smem_bytes()) ? 1 : 0;
     dim3 grid((unsigned)((P.total_rows + NROW - 1) / NROW));
@@ -201,12 +208,14 @@ template <class T, int LEN> struct FastList;
 #define X(LEN, ...)                                                                                         \
     template <class T> struct FastList<T, LEN> {                                                            \
         static void rows(hipgp_plan* pl, bool inv, RowsParams<T>& P, cudaStream_t st) { launch_rows_fast_t<T, __VA_ARGS__>(pl, inv, P, st); } \
+        static size_t rows_smem(long n_real) { return rows_fast_smem<T, __VA_ARGS__>(n_real); }                 \
         static void cols(hipgp_plan* pl, ColsParams<T>& P, long no, long B, cudaStream_t st) {         \
             if (!ColsBlkLaunch<T, LEN, __VA_ARGS__>::run(pl, P, no, B, st)) launch_cols_fast_t<T, LEN, __VA_ARGS__>(pl, P, no, B, st); } \
     };
 HIPGP_FAST_LIST(X)
 #undef X
 template <class T, int LEN> void launch_rows_fast_len(hipgp_plan* pl, bool inverse, RowsParams<T>& P, cudaStream_t st) { FastList<T, LEN>::rows(pl, inverse, P, st); }
+template <class T, int LEN> bool rows_fast_fits_len(long n_real) { return FastList<T, LEN>::rows_smem(n_real) <= kRowsFastSmemMax; }
 template <class T, int LEN> bool launch_cols_fast_len(hipgp_plan* pl, ColsParams<T>& P, long n_outer, long B, cudaStream_t st) {
     if (!cols_lane_aligned<T>(P)) throw Error("column pass: pointers / strides are not 16-byte aligned");
     FastList<T, LEN>::cols(pl, P, n_outer, B, st);

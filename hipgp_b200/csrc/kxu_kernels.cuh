@@ -310,9 +310,11 @@ __global__ void __launch_bounds__(256) doubly_diag_grad_kernel(const T* __restri
 }
 
 // grid (nchunk, B), block 256; op 0: dot(a,b) | op 1: x += al p, r -= al Ap, dot(r,r) | op 2: p = z + be p
+// (done: optional PCG early-exit flag, as in the fused passes)
 template <class T>
 __global__ void __launch_bounds__(256) vec_kernel(int op, T* x, T* r, const T* a, const T* b2, const double* s_num, const double* s_den,
-                                                  double* partial, long M, int nchunk) {
+                                                  double* partial, long M, int nchunk, const int* done) {
+    if (done && *done) return;
     const long bb = blockIdx.y;
     const long per = (M + nchunk - 1) / nchunk;
     const long lo = (long)blockIdx.x * per, hi = lo + per < M ? lo + per : M;
@@ -377,7 +379,8 @@ __global__ void __launch_bounds__(256) mf_colstats_kernel(const T* __restrict__ 
     dm[j] = a; lam[j] = l;
 }
 
-__global__ void vec_reduce_kernel(const double* partial, double* out, int nchunk, long B) {
+__global__ void vec_reduce_kernel(const double* partial, double* out, int nchunk, long B, const int* done) {
+    if (done && *done) return;
     const long bb = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (bb >= B) return;
     double t = 0;

@@ -3,6 +3,7 @@
 #include "plan_types.cuh"
 #include "setup_kernels.cuh"
 #include "kxu_kernels.cuh"
+#include "long1d_kernels.cuh"
 
 namespace hipgp {
 thread_local std::string g_err;
@@ -20,11 +21,36 @@ template <class T>
 static void pick_rows_tiling(long total_rows, int H, int* RB, int* RBP, int* nthreads) {
     int rb = 8;
     while (rb > 1 && (rows_smem<T>(H, rb + 1) > 96 * 1024 || total_rows < (long)rb * 148)) rb >>= 1;
-    if (rows_smem<T>(H, rb + 1) > 200 * 1024) throw Error("row axis too long for the shared-memory FFT (L = " + std::to_string(2 * H) + ")");
+    if (rows_smem<T>(H, rb + 1) > HIPGP_ROW_SMEM_MAX) throw Error("row axis too long for the shared-memory FFT (L = " + std::to_string(2 * H) + ")");
     *RB = rb; *RBP = rb == 1 ? 1 : rb + 1;
     long work = (long)H * rb / 8;
     *nthreads = work >= 256 ? 256 : (work >= 128 ? 128 : (work >= 64 ? 64 : 32));
 }
+
+// Does the row pass take a row of H complex bins in rows of up to n_real samples?  The specialised kernels need their tile
+// plus a side buffer of the real rows, the generic kernel two padded rows (pick_rows_tiling).
+template <class T>
+static bool row_pass_fits(int H, long n_real) {
+    switch (H) {
+#define X(LEN, ...) case LEN: return rows_fast_fits_len<T, LEN>(n_real);
+        HIPGP_FAST_LIST(X)
+#undef X
+        default: return rows_smem<T>(H, 2) <= HIPGP_ROW_SMEM_MAX;
+    }
+}
+// ... for every pass of a 1-D embedding of length L: the matvecs (rows of up to n_max samples, plan dtype) and the fp64
+// set-up forward of the whole embedding (forward_full)
+template <class T>
+static bool row_embedding_fits(int L, long n_max) { return row_pass_fits<T>(L / 2, n_max) && row_pass_fits<double>(L / 2, L); }
+
+// the four-step path of long 1-D embeddings (long1d_api.inl)
+template <class T> static LongGeom<T>& long_geom(hipgp_plan* pl, int which);
+template <class T> static void long_conv(hipgp_plan* pl, LongGeom<T>& g, const T* in, long n_in, T* out, long n_out, const void* spec,
+                                         int kind, long B, const int* done, cudaStream_t s);
+template <class T> static void long_build_spectrum(hipgp_plan* pl, bool wide, const double* col, DevBuf& dst, bool complex_spec, cudaStream_t s);
+static void long_dct1(hipgp_plan* pl, const double* in, double* out, bool normalise, cudaStream_t s);
+template <class T> static void long_pcg_begin(hipgp_plan* pl, const PcgDev& st, long B, bool precond, cudaStream_t s);
+template <class T> static void long_pcg_iterate(hipgp_plan* pl, const PcgDev& st, int niter, cudaStream_t s);
 
 template <class T> static bool aligned2(const void* p) { return ((uintptr_t)p % (2 * sizeof(T))) == 0; }
 
@@ -252,6 +278,11 @@ static const double* axis_cosmat(hipgp_plan* pl, int d, cudaStream_t s) {
     return b.as<double>();
 }
 
+// dct1_tile_kernel forms the cosine index (j k) mod N in 32-bit unsigned arithmetic
+static void dct1_tile_check(int md) {
+    if (md > 65536) throw Error("DCT-I set-up: an axis of " + std::to_string(md) + " points is beyond the tiled kernel (at most 65536)");
+}
+
 static void dct_all_axes(hipgp_plan* pl, const double* in, double* out, double* tmp, bool normalise, cudaStream_t s) {
     // separable DCT-I over the active axes; result always lands in `out`
     const double* src = in;
@@ -274,7 +305,7 @@ static void dct_all_axes(hipgp_plan* pl, const double* in, double* out, double* 
                 const int hk0 = (md + 1) / 2;
                 dim3 gs((unsigned)((hk0 + 63) / 64), (unsigned)((outer + 127) / 128), 2);
                 auto k = dct1_sym_kernel<true>; HIPGP_LAUNCH(k, gs, dim3(256), 0, s, src, dst, cw, md, inner, outer, scale, 0);
-            } else { auto k = dct1_tile_kernel<true>; HIPGP_LAUNCH(k, grid, dim3(256), 0, s, src, dst, tab, md, inner, outer, scale); }
+            } else { dct1_tile_check(md); auto k = dct1_tile_kernel<true>; HIPGP_LAUNCH(k, grid, dim3(256), 0, s, src, dst, tab, md, inner, outer, scale); }
         } else {
             // grid.z = outer index (<= 65535 for every supported grid: at most two leading axes of a 3-D grid)
             if (outer > 65535) throw Error("DCT set-up: more than 65535 outer slices");
@@ -284,7 +315,7 @@ static void dct_all_axes(hipgp_plan* pl, const double* in, double* out, double* 
                 const int hk0 = (md + 1) / 2, nty = (hk0 + 127) / 128;
                 dim3 gs((unsigned)((inner + 63) / 64), (unsigned)(2 * nty), (unsigned)outer);
                 auto k = dct1_sym_kernel<false>; HIPGP_LAUNCH(k, gs, dim3(256), 0, s, src, dst, cw, md, inner, outer, scale, nty);
-            } else { auto k = dct1_tile_kernel<false>; HIPGP_LAUNCH(k, grid, dim3(256), 0, s, src, dst, tab, md, inner, outer, scale); }
+            } else { dct1_tile_check(md); auto k = dct1_tile_kernel<false>; HIPGP_LAUNCH(k, grid, dim3(256), 0, s, src, dst, tab, md, inner, outer, scale); }
         }
         CK_LAUNCH();
         pl->launches++;
@@ -292,8 +323,15 @@ static void dct_all_axes(hipgp_plan* pl, const double* in, double* out, double* 
     }
 }
 
+// the DCT-I of set_first_row / ensure_wide: Bluestein on long 1-D plans, the tiled kernels otherwise
+static void dct1(hipgp_plan* pl, const double* in, double* out, double* tmp, bool normalise, cudaStream_t s) {
+    if (pl->long_n) long_dct1(pl, in, out, normalise, s);
+    else dct_all_axes(pl, in, out, tmp, normalise, s);
+}
+
 template <class T>
 static void build_spectrum(hipgp_plan* pl, bool wide, const double* col, DevBuf& dst, bool complex_spec, cudaStream_t s) {
+    if (wide ? pl->long_w : pl->long_n) { long_build_spectrum<T>(pl, wide, col, dst, complex_spec, s); return; }
     Geom<double>& g = wide ? pl->gw64 : pl->gn64;
     EmbedDims e{};
     e.D = g.D;
@@ -329,6 +367,7 @@ static void build_spectrum(hipgp_plan* pl, bool wide, const double* col, DevBuf&
 
 template <class T>
 static void ensure_geoms(hipgp_plan* pl, bool wide) {
+    if (wide ? pl->long_w : pl->long_n) return;      // four-step geometry instead, built on first use
     Geom<double>& g64 = wide ? pl->gw64 : pl->gn64;
     const int* L = wide ? pl->Lw : pl->Ln;
     if (!g64.built) g64.build(pl->D, L, &pl->dev_bytes);
@@ -355,7 +394,7 @@ static void set_first_row(hipgp_plan* pl, const void* column, double clampv, cud
         CK_LAUNCH(); pl->launches++;
     }
     // D = DCT-I(column), clamp, derive
-    dct_all_axes(pl, pl->colK.as<double>(), pl->tmpA.as<double>(), pl->tmpB.as<double>(), false, s);
+    dct1(pl, pl->colK.as<double>(), pl->tmpA.as<double>(), pl->tmpB.as<double>(), false, s);
     {
         auto k = clamp_derive_kernel<T>;
         HIPGP_LAUNCH(k, dim3(nb), dim3(256), 0, s, pl->tmpA.as<double>(), pl->Dm.as<double>(), pl->Dinv.as<double>(),
@@ -368,8 +407,8 @@ static void set_first_row(hipgp_plan* pl, const void* column, double clampv, cud
     pl->nclamped = hc[0];
     // first columns of C' (only when something was clamped or rounded: otherwise the column itself), C'^-1, C'^1/2
     if (pl->nclamped != 0 || sizeof(T) == 4)
-        dct_all_axes(pl, pl->Dm.as<double>(), pl->colK.as<double>(), pl->tmpB.as<double>(), true, s);
-    dct_all_axes(pl, pl->Dinv.as<double>(), pl->colG.as<double>(), pl->tmpB.as<double>(), true, s);
+        dct1(pl, pl->Dm.as<double>(), pl->colK.as<double>(), pl->tmpB.as<double>(), true, s);
+    dct1(pl, pl->Dinv.as<double>(), pl->colG.as<double>(), pl->tmpB.as<double>(), true, s);
     // (the first column of C'^1/2 belongs to the wide embedding: ensure_wide builds it on the first R^T / R)
     build_spectrum<T>(pl, false, pl->colK.as<double>(), pl->specK, false, s);
     build_spectrum<T>(pl, false, pl->colG.as<double>(), pl->specCinv, false, s);
@@ -386,7 +425,7 @@ static void ensure_wide(hipgp_plan* pl, cudaStream_t s) {
     bool real_ok = true;
     for (int d = 0; d < pl->D; ++d) if (pl->Lw[d] < 2 * pl->N[d] - 1) real_ok = false;
     pl->wide_real = real_ok;
-    dct_all_axes(pl, pl->Dsqrt.as<double>(), pl->colS.as<double>(), pl->tmpB.as<double>(), true, s);
+    dct1(pl, pl->Dsqrt.as<double>(), pl->colS.as<double>(), pl->tmpB.as<double>(), true, s);
     build_spectrum<T>(pl, true, pl->colS.as<double>(), pl->specW, !real_ok, s);
     pl->have_wide = true;
 }
@@ -403,7 +442,6 @@ static void matvec(hipgp_plan* pl, int mode, const void* in, void* out, long B, 
     ff.mode = RF_PLAIN; ff.in = in; fi.mode = RI_PLAIN; fi.out = out;
     const bool wide = (mode == HIPGP_MV_RT || mode == HIPGP_MV_R);
     if (wide) ensure_wide<T>(pl, s);
-    Geom<T>& g = geom(pl, wide, Tag<T>());
     int n_in[3], n_out[3];
     for (int d = 0; d < pl->D; ++d) {
         n_in[d] = mode == HIPGP_MV_R ? pl->N[d] : pl->m[d];
@@ -417,7 +455,11 @@ static void matvec(hipgp_plan* pl, int mode, const void* in, void* out, long B, 
         case HIPGP_MV_R: spec = pl->specW.p; kind = pl->wide_real ? SPEC_REAL : SPEC_CPLX_CONJ; break;
         default: throw Error("unknown matvec mode");
     }
-    run_pipeline<T>(pl, g, n_in, n_out, spec, kind, B, ff, fi, null_state(), false, s);
+    if (wide ? pl->long_w : pl->long_n) {
+        long_conv<T>(pl, long_geom<T>(pl, wide ? 1 : 0), (const T*)in, n_in[0], (T*)out, n_out[0], spec, kind, B, nullptr, s);
+        return;
+    }
+    run_pipeline<T>(pl, geom(pl, wide, Tag<T>()), n_in, n_out, spec, kind, B, ff, fi, null_state(), false, s);
 }
 
 template <class T>
@@ -470,9 +512,6 @@ static void pcg_begin(hipgp_plan* pl, const void* b, void* x, long B, double tol
     const long M = pl->M;
     PcgDev st = pcg_state<T>(pl, B, tol, !precond);
     if (!pl->pinned) CK(cudaMallocHost(&pl->pinned, 64));
-    Geom<T>& g = geom(pl, false, Tag<T>());
-    int nn[3];
-    for (int d = 0; d < pl->D; ++d) nn[d] = pl->m[d];
     T* r = pl->vr.as<T>(); T* z = precond ? pl->vz.as<T>() : r;
     // x = 0 ; r = b - A(0) = b   (cg.py:58-59; the reference spends a matvec on the zero vector)
     CK(cudaMemsetAsync(x, 0, sizeof(T) * (size_t)(B * M), s));
@@ -481,9 +520,13 @@ static void pcg_begin(hipgp_plan* pl, const void* b, void* x, long B, double tol
     CK(cudaMemsetAsync(st.flags, 0, sizeof(int) * 4, s));
     CK(cudaMemsetAsync(reinterpret_cast<char*>(st.flags) + 2 * sizeof(int), 1, 1, s));
     RowsFusion ff, fi;
-    if (precond) {   // z = P r ; zr = z.r
+    if (pl->long_n) {
+        long_pcg_begin<T>(pl, st, B, precond, s);
+    } else if (precond) {   // z = P r ; zr = z.r
+        int nn[3];
+        for (int d = 0; d < pl->D; ++d) nn[d] = pl->m[d];
         ff.mode = RF_PLAIN; ff.in = r; fi.mode = RI_DOT; fi.dot_kind = DOT_ZR; fi.out = z; fi.v0 = r;
-        run_pipeline<T>(pl, g, nn, nn, pl->specCinv.p, SPEC_REAL, B, ff, fi, st, false, s);
+        run_pipeline<T>(pl, geom(pl, false, Tag<T>()), nn, nn, pl->specCinv.p, SPEC_REAL, B, ff, fi, st, false, s);
     } else {         // z = r ; zr = r.r
         launch_vec<T>(pl, RF_SELFDOT, st, B, r, nullptr, nullptr, nullptr, s);
     }
@@ -497,6 +540,7 @@ static void pcg_iterate(hipgp_plan* pl, int niter, cudaStream_t s) {
     const long B = pl->run_B;
     const bool precond = pl->run_precond;
     PcgDev st = pcg_state<T>(pl, B, pl->run_tol, !precond);
+    if (pl->long_n) { long_pcg_iterate<T>(pl, st, niter, s); return; }
     Geom<T>& g = geom(pl, false, Tag<T>());
     int nn[3];
     for (int d = 0; d < pl->D; ++d) nn[d] = pl->m[d];
@@ -608,11 +652,30 @@ int hipgp_plan_create(int ndim, const int64_t* m, int dtype, int device, hipgp_p
     }
     if (D == 0) { D = 1; pl->m[0] = 1; pl->N[0] = 1; }
     pl->D = D;
-    for (int d = 0; d < D; ++d) {
-        const bool row = (d == D - 1);
-        pl->Ln[d] = choose_length(2L * pl->m[d] - 1, row);
-        pl->Lw[d] = choose_length((long)pl->N[d] + pl->m[d] - 1, row);
-    }
+    try {
+        for (int d = 0; d < D; ++d) {
+            const bool row = (d == D - 1);
+            pl->Ln[d] = choose_length(2L * pl->m[d] - 1, row);
+            pl->Lw[d] = choose_length((long)pl->N[d] + pl->m[d] - 1, row);
+        }
+        // a 1-D embedding whose row pass would not fit shared memory takes the four-step path, at a length L1 * L2
+        if (D == 1) {
+            const long m0 = pl->m[0], N0 = pl->N[0];
+            auto fits = [&](int L, long n_max) { return dtype == HIPGP_F32 ? row_embedding_fits<float>(L, n_max) : row_embedding_fits<double>(L, n_max); };
+            auto split = [&](long n, int which, int* L) {
+                int* f = pl->lsplit[which];
+                if (!long_split(n, &f[0], &f[1]))
+                    throw Error("1-D grid of " + std::to_string(m0) + " points is too long: the four-step path reaches " +
+                                std::to_string((long)kLongMaxFactor * kLongMaxFactor) + "-point transforms (m <= " +
+                                std::to_string(((long)kLongMaxFactor * kLongMaxFactor + 5) / 4) + ")");
+                if (L) *L = f[0] * f[1];
+            };
+            pl->long_n = !fits(pl->Ln[0], m0);
+            pl->long_w = pl->long_n || !fits(pl->Lw[0], N0);
+            if (pl->long_n) { split(2 * m0 - 1, 0, &pl->Ln[0]); split(2 * N0 - 1, 2, nullptr); }
+            if (pl->long_w) split(N0 + m0 - 1, 1, &pl->Lw[0]);
+        }
+    } catch (...) { delete pl; throw; }
     *out = pl;
     API_END
 }
@@ -622,6 +685,8 @@ int hipgp_plan_destroy(hipgp_plan* pl) {
     if (!pl) return 0;
     size_t* t = &pl->dev_bytes;
     pl->gn32.release(t); pl->gw32.release(t); pl->gn64.release(t); pl->gw64.release(t);
+    pl->ln32.release(t); pl->lw32.release(t); pl->ln64.release(t); pl->lw64.release(t); pl->lb64.release(t);
+    pl->bluA.release(t); pl->bluSpec.release(t);
     for (DevBuf* b : {&pl->specK, &pl->specCinv, &pl->specW, &pl->Dm, &pl->Dinv, &pl->Dsqrt, &pl->colK, &pl->colG, &pl->colS,
                       &pl->tmpA, &pl->tmpB, &pl->counts, &pl->W1, &pl->W2, &pl->vr, &pl->vp, &pl->vz, &pl->vAp,
                       &pl->partial, &pl->scal, &pl->cnt, &pl->flags, &pl->stage_in, &pl->stage_out, &pl->corrU, &pl->corrV, &pl->corrS,
@@ -936,6 +1001,7 @@ int hipgp_plan_launch_count(const hipgp_plan* pl, int64_t* launches) { API_BEGIN
 }  // extern "C"
 
 #include "vec_api.inl"
+#include "long1d_api.inl"
 #include "kxu_api.inl"
 #include "corr_api.inl"
 #include "block_api.inl"

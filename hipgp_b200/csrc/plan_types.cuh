@@ -99,6 +99,33 @@ inline bool is_smooth(long n) {
     return n == 1;
 }
 
+// Shared-memory budgets of the row passes: the generic kernel (pick_rows_tiling, two padded rows at least) and the
+// specialised kernels (tile + side buffer).  A 1-D embedding whose row pass would exceed them takes the four-step path of
+// long1d_api.inl instead.  The test-only emulation build lowers HIPGP_ROW_SMEM_MAX with -D to run that path at small sizes.
+#ifndef HIPGP_ROW_SMEM_MAX
+#define HIPGP_ROW_SMEM_MAX (200 * 1024)
+#endif
+constexpr size_t kRowsFastSmemMax = 227 * 1024;
+// Four-step lengths L = L1 * L2: both factors from HIPGP_FAST_LIST and at most this long, so that one line (fp64: 64 KB)
+// and its neighbours fit a CTA's shared memory.
+constexpr int kLongMaxFactor = 4096;
+
+// smallest L = L1 * L2 >= n with L1 <= L2 both in HIPGP_FAST_LIST (<= kLongMaxFactor); among equal L the most balanced split
+inline bool long_split(long n, int* L1, int* L2) {
+    std::vector<int> f;
+#define X(LEN, ...) if (LEN <= kLongMaxFactor) f.push_back(LEN);
+    HIPGP_FAST_LIST(X)
+#undef X
+    long best = -1;
+    for (int a : f)
+        for (int b : f) {
+            const long L = (long)a * b;
+            if (a > b || L < n) continue;
+            if (best < 0 || L < best || (L == best && a > *L1)) { best = L; *L1 = a; *L2 = b; }
+        }
+    return best > 0;
+}
+
 // smallest-cost 2^a 3^b 5^c length >= n (even when `even`), searched in [n, 2n]
 inline int choose_length(long n, bool even) {
     if (n < 2) n = 2;
@@ -252,6 +279,27 @@ struct Geom {
     void release(size_t* total) { for (auto& f : fcol) f.release(total); frow.release(total); twL.release(total); twLp.release(total); part.release(total); pairq.release(total); pairs.release(total); pairw.release(total); quadq.release(total); quadw.release(total); built = false; }
 };
 
+// four-step geometry of a long 1-D embedding (long1d_kernels.cuh): the two line FFTs and the twiddle tables, fp64-computed
+template <class T>
+struct LongGeom {
+    int L1 = 0, L2 = 0;
+    LineFftHost<T> f1, f2;
+    DevBuf twh, twl;
+    bool built = false;
+    void build(int L1_, int L2_, size_t* total) {
+        L1 = L1_; L2 = L2_;
+        f1.build(L1, total); f2.build(L2, total);
+        std::vector<cplx<T>> h(L1), l(L2);
+        for (int j = 0; j < L1; ++j) { const double a = -2.0 * M_PI * (double)j / (double)L1; h[j].x = (T)std::cos(a); h[j].y = (T)std::sin(a); }
+        for (int j = 0; j < L2; ++j) { const double a = -2.0 * M_PI * (double)j / ((double)L1 * L2); l[j].x = (T)std::cos(a); l[j].y = (T)std::sin(a); }
+        twh.ensure(sizeof(cplx<T>) * L1, total); twl.ensure(sizeof(cplx<T>) * L2, total);
+        CK(cudaMemcpy(twh.p, h.data(), sizeof(cplx<T>) * L1, cudaMemcpyHostToDevice));
+        CK(cudaMemcpy(twl.p, l.data(), sizeof(cplx<T>) * L2, cudaMemcpyHostToDevice));
+        built = true;
+    }
+    void release(size_t* total) { f1.release(total); f2.release(total); twh.release(total); twl.release(total); built = false; }
+};
+
 struct RowsFusion {
     int mode = 0, dot_kind = 0, do_fft = 1;
     const void* in = nullptr; void* out = nullptr; void* v0 = nullptr; void* v1 = nullptr; const void* v2 = nullptr;
@@ -279,6 +327,14 @@ struct hipgp_plan {
 
     Geom<float> gn32, gw32;    // narrow (K, Cinv) / wide (RT, R) geometries in the plan dtype
     Geom<double> gn64, gw64;   // fp64 geometries (set-up always runs in fp64; also the fp64 plan's own)
+    // 1-D embeddings too long for the row pass run the four-step path (long1d_api.inl): narrow / wide, each decided on its
+    // own; lsplit = (L1, L2) of the narrow, wide and Bluestein (DCT-I set-up, only when the narrow one is long) lengths
+    bool long_n = false, long_w = false;
+    int lsplit[3][2] = {{0, 0}, {0, 0}, {0, 0}};
+    LongGeom<float> ln32, lw32;
+    LongGeom<double> ln64, lw64, lb64;
+    DevBuf bluA, bluSpec;                  // Bluestein work array and the chirp's spectrum (built once per plan)
+    bool have_blu = false, long_first = false;
     DevBuf specK, specCinv, specW;         // stored spectra (plan dtype; specW complex)
     DevBuf Dm, Dinv, Dsqrt, colK, colG, colS, tmpA, tmpB, counts;   // fp64 set-up arrays (M each)
     DevBuf W1, W2;                         // frequency-domain workspace
@@ -332,4 +388,5 @@ struct hipgp_plan {
 namespace hipgp {
 template <class T, int LEN> void launch_rows_fast_len(hipgp_plan* pl, bool inverse, RowsParams<T>& P, cudaStream_t st);
 template <class T, int LEN> bool launch_cols_fast_len(hipgp_plan* pl, ColsParams<T>& P, long n_outer, long B, cudaStream_t st);   // false: lanes not 16-byte aligned
+template <class T, int LEN> bool rows_fast_fits_len(long n_real);   // does the row pass of this length fit rows of n_real samples?
 }
