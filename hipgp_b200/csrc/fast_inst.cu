@@ -5,7 +5,7 @@
 namespace hipgp {
 #define INST(T, LEN)                                                                                            \
     template void launch_rows_fast_len<T, LEN>(hipgp_plan*, bool, RowsParams<T>&, cudaStream_t);                \
-    template bool launch_cols_fast_len<T, LEN>(hipgp_plan*, ColsParams<T>&, long, long, cudaStream_t);            \
+    template void launch_cols_fast_len<T, LEN>(hipgp_plan*, ColsParams<T>&, long, long, cudaStream_t);            \
     template bool rows_fast_fits_len<T, LEN>(long);
 #ifndef HIPGP_INST_GROUP
 #define X(LEN, ...) INST(float, LEN) INST(double, LEN)

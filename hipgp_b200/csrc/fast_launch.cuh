@@ -216,9 +216,8 @@ HIPGP_FAST_LIST(X)
 #undef X
 template <class T, int LEN> void launch_rows_fast_len(hipgp_plan* pl, bool inverse, RowsParams<T>& P, cudaStream_t st) { FastList<T, LEN>::rows(pl, inverse, P, st); }
 template <class T, int LEN> bool rows_fast_fits_len(long n_real) { return FastList<T, LEN>::rows_smem(n_real) <= kRowsFastSmemMax; }
-template <class T, int LEN> bool launch_cols_fast_len(hipgp_plan* pl, ColsParams<T>& P, long n_outer, long B, cudaStream_t st) {
+template <class T, int LEN> void launch_cols_fast_len(hipgp_plan* pl, ColsParams<T>& P, long n_outer, long B, cudaStream_t st) {
     if (!cols_lane_aligned<T>(P)) throw Error("column pass: pointers / strides are not 16-byte aligned");
     FastList<T, LEN>::cols(pl, P, n_outer, B, st);
-    return true;
 }
 }  // namespace hipgp

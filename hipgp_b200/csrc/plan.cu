@@ -39,7 +39,7 @@ static bool row_pass_fits(int H, long n_real) {
     }
 }
 // ... for every pass of a 1-D embedding of length L: the matvecs (rows of up to n_max samples, plan dtype) and the fp64
-// set-up forward of the whole embedding (forward_full)
+// set-up forward of the whole embedding (build_spectrum)
 template <class T>
 static bool row_embedding_fits(int L, long n_max) { return row_pass_fits<T>(L / 2, n_max) && row_pass_fits<double>(L / 2, L); }
 
@@ -64,25 +64,14 @@ static bool launch_rows_fast(hipgp_plan* pl, bool inverse, RowsParams<T>& P, cud
     }
 }
 
-// Does every pass of this geometry have a specialised kernel?  fp32 pipelines keep the frequency workspace in lane
-// layout (lane_fft.cuh), which the generic kernels do not read, so an fp32 pipeline is all specialised or all generic;
-// fp64 lanes are plain interleaved complex numbers and the choice is made kernel by kernel.
 template <class T>
-static bool geom_allows_fast(const Geom<T>& g) {
-    if (sizeof(T) == 8) return true;
-    if (fast_radices(g.H).empty()) return false;
-    for (int d = 0; d + 1 < g.D; ++d) if (fast_radices(g.L[d]).empty()) return false;
-    return true;
-}
-
-template <class T>
-static void launch_rows(hipgp_plan* pl, bool inverse, RowsParams<T>& P, cudaStream_t st, bool allow_fast = true) {
+static void launch_rows(hipgp_plan* pl, const Geom<T>& g, bool inverse, RowsParams<T>& P, cudaStream_t st) {
     P.vec_ok = (aligned2<T>(P.in) && aligned2<T>(P.out) && aligned2<T>(P.v0) && aligned2<T>(P.v1) && aligned2<T>(P.v2)) ? 1 : 0;
     {
         auto a16 = [](const void* q) { return ((uintptr_t)q % 16) == 0; };
         P.vec16_ok = (a16(P.in) && a16(P.out) && a16(P.v0) && a16(P.v1) && a16(P.v2)) ? 1 : 0;
     }
-    if (allow_fast && P.do_fft && launch_rows_fast<T>(pl, inverse, P, st)) return;
+    if (g.fast && launch_rows_fast<T>(pl, inverse, P, st)) return;
     int nth;
     pick_rows_tiling<T>(P.total_rows, P.H, &P.RB, &P.RBP, &nth);
     const size_t smem = rows_smem<T>(P.H, P.RBP);
@@ -105,7 +94,7 @@ static void launch_rows(hipgp_plan* pl, bool inverse, RowsParams<T>& P, cudaStre
 template <class T>
 static bool launch_cols_fast(hipgp_plan* pl, ColsParams<T>& P, long n_outer, long B, cudaStream_t st) {
     switch (P.f.Ln) {
-#define X(LEN, ...) case LEN: return launch_cols_fast_len<T, LEN>(pl, P, n_outer, B, st);
+#define X(LEN, ...) case LEN: launch_cols_fast_len<T, LEN>(pl, P, n_outer, B, st); return true;
         HIPGP_FAST_LIST(X)
 #undef X
         default: return false;
@@ -113,8 +102,8 @@ static bool launch_cols_fast(hipgp_plan* pl, ColsParams<T>& P, long n_outer, lon
 }
 
 template <class T>
-static void launch_cols(hipgp_plan* pl, ColsParams<T>& P, long n_outer, long B, cudaStream_t st, bool allow_fast = true) {
-    if (allow_fast && launch_cols_fast<T>(pl, P, n_outer, B, st)) return;
+static void launch_cols(hipgp_plan* pl, const Geom<T>& g, ColsParams<T>& P, long n_outer, long B, cudaStream_t st) {
+    if (g.fast && launch_cols_fast<T>(pl, P, n_outer, B, st)) return;
     const int L = P.f.Ln;
     int tb = sizeof(T) == 4 ? 16 : 8;
     while (tb > 1 && sizeof(cplx<T>) * (size_t)L * (tb + 1) > 100 * 1024) tb >>= 1;
@@ -135,23 +124,63 @@ static void launch_cols(hipgp_plan* pl, ColsParams<T>& P, long n_outer, long B, 
     pl->launches++;
 }
 
-// the row-axis tables of a geometry
+static PcgDev null_state() { PcgDev st{}; return st; }
+static RowsFusion plain_in(const void* in) { RowsFusion f; f.mode = RF_PLAIN; f.in = in; return f; }
+static RowsFusion plain_out(void* out) { RowsFusion f; f.mode = RI_PLAIN; f.out = out; return f; }
+
+// One row pass over B batch entries of `nrows` rows each.  Forward: real rows of n_real samples (f.in, or the operands of
+// the fused update f) -> half spectra in W.  Inverse: W -> real rows of n_real samples (f.out, f.v0), after applying the
+// 1-D spectrum `spec` when there is one.  Batch entry b owns W_rows >= nrows rows of W, g.P complex elements each.
 template <class T>
-static void rows_geom(RowsParams<T>& R, Geom<T>& g) {
+static void run_rows(hipgp_plan* pl, Geom<T>& g, bool inverse, long nrows, cplx<T>* W, long W_rows, long B, int n_real,
+                     const RowsFusion& f, const PcgDev& st, cudaStream_t s, const void* spec = nullptr, int spec_kind = SPEC_NONE) {
+    RowsParams<T> R{};
     R.L = g.L[g.D - 1]; R.H = g.H; R.W_pitch = g.P;
     R.f = g.frow.dev; R.twL = g.twL.template as<cplx<T>>(); R.twLp = g.twLp.template as<cplx<T>>();
     R.part = g.part.template as<int>(); R.pairq = g.pairq.template as<int>();
     R.pairs = g.pairs.template as<int>(); R.pairw = g.pairw.template as<cplx<T>>(); R.npair0 = g.npair0;
     R.quadq = g.quadq.template as<int>(); R.quadw = g.quadw.template as<cplx<T>>(); R.nquad = g.nquad;
+    R.in = (const T*)f.in; R.out = (T*)f.out; R.v0 = (T*)f.v0; R.v1 = (T*)f.v1; R.v2 = (const T*)f.v2;
+    R.mode = f.mode; R.dot_kind = f.dot_kind; R.do_fft = 1; R.st = st; R.spec = spec; R.spec_kind = spec_kind;
+    R.W = W; R.W_rows = (int)W_rows; R.total_rows = B * nrows; R.nrows = (int)nrows; R.n_real = n_real;
+    launch_rows<T>(pl, g, inverse, R, s);
 }
 
-// workspace requirement (complex elements) for a pipeline with the given extents
-static void ws_elems(int D, const int* L, long P, const int* n_in, const int* n_out, long B, long* w1, long* w2) {
-    if (D == 1) { *w1 = B * P; *w2 = 0; return; }
-    if (D == 2) { *w1 = B * std::max(n_in[0], n_out[0]) * P; *w2 = 0; return; }
-    const long R01 = std::max((long)n_in[0] * n_in[1], (long)n_out[0] * n_out[1]);
-    const long R0 = std::max(n_in[0], n_out[0]);
-    *w1 = B * R01 * P; *w2 = B * R0 * (long)L[1] * P;
+// A buffer of the column passes: batch entries `bstride` complex elements apart, each holding n[0] (x n[1]) rows along
+// the leading axes, row-major.
+template <class T> struct ColBuf { cplx<T>* p; long bstride; const int* n; };
+
+// The column passes of the leading D - 1 axes from src to dst, over B batch entries of rows of `pitch` complex elements
+// whose first `bins` are transformed.  chain CM_FWD: forward, src zero-padded to L, dst holds all L[0] (x L[1]) rows;
+// CM_INV: inverse, src holds all L rows (and is overwritten), dst gets its own extents; CM_FUSED: forward, times `spec` on
+// axis 0, inverse (3-D: through W2[b][max n0][L1][pitch]).  done: optional PCG early-exit flag.
+template <class T>
+static void run_cols(hipgp_plan* pl, Geom<T>& g, int chain, const ColBuf<T>& src, const ColBuf<T>& dst, long pitch, long bins,
+                     long B, const void* spec, int spec_kind, const int* done, cudaStream_t s) {
+    if (g.D == 1) return;
+    const long plane = (long)g.L[1] * pitch;      // 3-D: an [L1][pitch] plane, the lines of the axis-0 pass
+    auto pass = [&](int axis, int mode, const ColBuf<T>& in, const ColBuf<T>& out) {
+        const bool rows = axis == g.D - 2;
+        ColsParams<T> C{};
+        C.in = in.p; C.out = out.p; C.f = g.fcol[axis].dev; C.mode = mode; C.done_flag = done;
+        C.n_in = (mode == CM_INV ? dst : src).n[axis]; C.n_out = (mode == CM_FWD ? src : dst).n[axis];
+        C.inner = rows ? bins : plane; C.pitch = rows ? pitch : plane;
+        C.in_bstride = in.bstride; C.out_bstride = out.bstride;
+        if (axis == 1) { C.in_ostride = in.n[1] * pitch; C.out_ostride = out.n[1] * pitch; }
+        if (mode == CM_FUSED) { C.spec = spec; C.spec_kind = spec_kind; }
+        launch_cols<T>(pl, g, C, axis == 1 ? (mode == CM_FWD ? src : dst).n[0] : 1, B, s);
+    };
+    if (g.D == 2) { pass(0, chain, src, dst); return; }
+    // 3-D: axis 1 forward into a buffer of L1 rows per plane, axis 0 in place on it, axis 1 inverse out of it
+    ColBuf<T> mid = chain == CM_FWD ? dst : src;
+    const int mid_n[2] = {std::max(src.n[0], dst.n[0]), g.L[1]};
+    if (chain == CM_FUSED) {
+        pl->W2.ensure(sizeof(cplx<T>) * (size_t)(B * mid_n[0] * plane), &pl->dev_bytes);
+        mid = {pl->W2.as<cplx<T>>(), mid_n[0] * plane, mid_n};
+    }
+    if (chain != CM_INV) pass(1, CM_FWD, src, mid);
+    pass(0, chain, mid, mid);
+    if (chain != CM_FWD) pass(1, CM_INV, mid, dst);
 }
 
 // The pruned D-dimensional circular convolution:  out = crop_{n_out} IFFT( spec * FFT pad_{n_in} in ).
@@ -159,93 +188,18 @@ template <class T>
 static void run_pipeline(hipgp_plan* pl, Geom<T>& g, const int* n_in, const int* n_out, const void* spec, int spec_kind,
                          long B, const RowsFusion& ff, const RowsFusion& fi, const PcgDev& st, bool gated, cudaStream_t s) {
     const int D = g.D;
-    long w1, w2;
-    ws_elems(D, g.L, g.P, n_in, n_out, B, &w1, &w2);
-    pl->W1.ensure(sizeof(cplx<T>) * (size_t)w1, &pl->dev_bytes);
-    if (w2) pl->W2.ensure(sizeof(cplx<T>) * (size_t)w2, &pl->dev_bytes);
-    cplx<T>* W1 = pl->W1.as<cplx<T>>();
-    cplx<T>* W2 = pl->W2.as<cplx<T>>();
-    const long P = g.P;
-    const int* done = gated ? st.flags : nullptr;
-    const bool fast = geom_allows_fast(g);
-
     long rows_in = 1, rows_out = 1;
     for (int d = 0; d + 1 < D; ++d) { rows_in *= n_in[d]; rows_out *= n_out[d]; }
     const long Wrows = std::max(rows_in, rows_out);
-
-    RowsParams<T> R{};
-    rows_geom(R, g);
-    R.W = W1; R.W_rows = (int)Wrows; R.st = st;
-    // forward rows
-    R.in = (const T*)ff.in; R.v0 = (T*)ff.v0; R.v1 = (T*)ff.v1; R.v2 = (const T*)ff.v2;
-    R.mode = ff.mode; R.do_fft = 1; R.total_rows = B * rows_in; R.nrows = (int)rows_in; R.n_real = n_in[D - 1];
-    R.spec = nullptr; R.spec_kind = SPEC_NONE;
-    launch_rows<T>(pl, false, R, s, fast);
-
-    if (D == 2) {
-        ColsParams<T> C{};
-        C.in = W1; C.out = W1; C.n_in = n_in[0]; C.n_out = n_out[0]; C.inner = g.H + 1; C.pitch = P;
-        C.in_ostride = C.out_ostride = 0; C.in_bstride = C.out_bstride = Wrows * P;
-        C.f = g.fcol[0].dev; C.mode = CM_FUSED; C.spec = spec; C.spec_kind = spec_kind; C.done_flag = done;
-        launch_cols<T>(pl, C, 1, B, s, fast);
-    } else if (D == 3) {
-        const long R0 = std::max(n_in[0], n_out[0]);
-        const long L1 = g.L[1];
-        ColsParams<T> C{};
-        C.done_flag = done; C.spec = nullptr; C.spec_kind = SPEC_NONE;
-        // axis 1 forward: W1[b][i0][n_in1][P] -> W2[b][i0][L1][P]
-        C.in = W1; C.out = W2; C.n_in = n_in[1]; C.n_out = n_in[1]; C.inner = g.H + 1; C.pitch = P;
-        C.in_ostride = (long)n_in[1] * P; C.in_bstride = Wrows * P; C.out_ostride = L1 * P; C.out_bstride = R0 * L1 * P;
-        C.f = g.fcol[1].dev; C.mode = CM_FWD;
-        launch_cols<T>(pl, C, n_in[0], B, s, fast);
-        // axis 0 fused, in place on W2
-        C.in = W2; C.out = W2; C.n_in = n_in[0]; C.n_out = n_out[0]; C.inner = L1 * P; C.pitch = L1 * P;
-        C.in_ostride = C.out_ostride = 0; C.in_bstride = C.out_bstride = R0 * L1 * P;
-        C.f = g.fcol[0].dev; C.mode = CM_FUSED; C.spec = spec; C.spec_kind = spec_kind;
-        launch_cols<T>(pl, C, 1, B, s, fast);
-        // axis 1 inverse: W2 -> W1[b][i0][n_out1][P]
-        C.in = W2; C.out = W1; C.n_in = n_out[1]; C.n_out = n_out[1]; C.inner = g.H + 1; C.pitch = P;
-        C.in_ostride = L1 * P; C.in_bstride = R0 * L1 * P; C.out_ostride = (long)n_out[1] * P; C.out_bstride = Wrows * P;
-        C.f = g.fcol[1].dev; C.mode = CM_INV; C.spec = nullptr; C.spec_kind = SPEC_NONE;
-        launch_cols<T>(pl, C, n_out[0], B, s, fast);
-    }
-
-    // inverse rows
-    R.out = (T*)fi.out; R.v0 = (T*)fi.v0; R.mode = fi.mode; R.dot_kind = fi.dot_kind;
-    R.total_rows = B * rows_out; R.nrows = (int)rows_out; R.n_real = n_out[D - 1];
-    if (D == 1) { R.spec = spec; R.spec_kind = spec_kind; }
-    launch_rows<T>(pl, true, R, s, fast);
-}
-
-// forward-only transform of a real (L_0..L_{D-1}) fp64 array into W1 (raw spectrum, pipeline layout)
-static void forward_full(hipgp_plan* pl, Geom<double>& g, const double* h, cudaStream_t s) {
-    const int D = g.D;
-    long rows = 1;
-    for (int d = 0; d + 1 < D; ++d) rows *= g.L[d];
-    pl->W1.ensure(sizeof(cplx<double>) * (size_t)rows * g.P, &pl->dev_bytes);
-    cplx<double>* W = pl->W1.as<cplx<double>>();
-    RowsParams<double> R{};
-    rows_geom(R, g);
-    R.in = h; R.W = W; R.W_rows = (int)rows; R.mode = RF_PLAIN; R.do_fft = 1;
-    R.total_rows = rows; R.nrows = (int)rows; R.n_real = g.L[D - 1];
-    launch_rows<double>(pl, false, R, s);
-    if (D >= 2) {
-        ColsParams<double> C{};
-        C.in = W; C.out = W; C.mode = CM_FWD; C.done_flag = nullptr; C.spec_kind = SPEC_NONE;
-        if (D == 3) {
-            C.n_in = C.n_out = g.L[1]; C.inner = g.H + 1; C.pitch = g.P;
-            C.in_ostride = C.out_ostride = (long)g.L[1] * g.P; C.in_bstride = C.out_bstride = 0;
-            C.f = g.fcol[1].dev;
-            launch_cols<double>(pl, C, g.L[0], 1, s);
-            C.n_in = C.n_out = g.L[0]; C.inner = (long)g.L[1] * g.P; C.pitch = (long)g.L[1] * g.P;
-            C.in_ostride = C.out_ostride = 0; C.f = g.fcol[0].dev;
-            launch_cols<double>(pl, C, 1, 1, s);
-        } else {
-            C.n_in = C.n_out = g.L[0]; C.inner = g.H + 1; C.pitch = g.P;
-            C.in_ostride = C.out_ostride = 0; C.in_bstride = C.out_bstride = 0; C.f = g.fcol[0].dev;
-            launch_cols<double>(pl, C, 1, 1, s);
-        }
-    }
+    pl->W1.ensure(sizeof(cplx<T>) * (size_t)(B * Wrows * g.P), &pl->dev_bytes);
+    cplx<T>* W1 = pl->W1.as<cplx<T>>();
+    run_rows<T>(pl, g, false, rows_in, W1, Wrows, B, n_in[D - 1], ff, st, s);
+    run_cols<T>(pl, g, CM_FUSED, {W1, Wrows * g.P, n_in}, {W1, Wrows * g.P, n_out}, g.P, g.H + 1, B, spec, spec_kind,
+                gated ? st.flags : nullptr, s);
+    // the inverse pass's alignment flags (vec_ok, vec16_ok) cover the forward pass's operands too
+    RowsFusion fo = fi;
+    fo.in = ff.in; fo.v1 = ff.v1; fo.v2 = ff.v2;
+    run_rows<T>(pl, g, true, rows_out, W1, Wrows, B, n_out[D - 1], fo, st, s, D == 1 ? spec : nullptr, D == 1 ? spec_kind : SPEC_NONE);
 }
 
 // cos(pi t / (m-1)), t in [0, 2(m-1)), per active axis: built once per plan (the grid never changes), no per-call copies
@@ -350,17 +304,21 @@ static void build_spectrum(hipgp_plan* pl, bool wide, const double* col, DevBuf&
         HIPGP_LAUNCH(k, dim3(nb), dim3(256), 0, s, col, pl->tmpB.as<double>(), e);
         CK_LAUNCH(); pl->launches++;
     }
-    forward_full(pl, g, pl->tmpB.as<double>(), s);
+    // forward transform of the embedded column into W1 (raw spectrum, pipeline layout)
     const long n = g.spec_elems();
+    pl->W1.ensure(sizeof(cplx<double>) * (size_t)n, &pl->dev_bytes);
+    cplx<double>* W1 = pl->W1.as<cplx<double>>();
+    run_rows<double>(pl, g, false, n / g.P, W1, n / g.P, 1, g.L[g.D - 1], plain_in(pl->tmpB.as<double>()), null_state(), s);
+    run_cols<double>(pl, g, CM_FWD, {W1, 0, g.L}, {W1, 0, g.L}, g.P, g.H + 1, 1, nullptr, SPEC_NONE, nullptr, s);
     double scale = 0.25;
     for (int d = 0; d < g.D; ++d) scale /= (double)g.L[d];
     const unsigned nblk = (unsigned)((n + 255) / 256);
     if (complex_spec) {
         dst.ensure(sizeof(cplx<T>) * (size_t)n, &pl->dev_bytes);
-        auto k = store_spec_cplx_kernel<T>; HIPGP_LAUNCH(k, dim3(nblk), dim3(256), 0, s, pl->W1.as<cplx<double>>(), dst.as<cplx<T>>(), n, scale);
+        auto k = store_spec_cplx_kernel<T>; HIPGP_LAUNCH(k, dim3(nblk), dim3(256), 0, s, W1, dst.as<cplx<T>>(), n, scale);
     } else {
         dst.ensure(sizeof(T) * (size_t)n, &pl->dev_bytes);
-        auto k = store_spec_real_kernel<T>; HIPGP_LAUNCH(k, dim3(nblk), dim3(256), 0, s, pl->W1.as<cplx<double>>(), dst.as<T>(), n, scale);
+        auto k = store_spec_real_kernel<T>; HIPGP_LAUNCH(k, dim3(nblk), dim3(256), 0, s, W1, dst.as<T>(), n, scale);
     }
     CK_LAUNCH(); pl->launches++;
 }
@@ -430,16 +388,12 @@ static void ensure_wide(hipgp_plan* pl, cudaStream_t s) {
     pl->have_wide = true;
 }
 
-static PcgDev null_state() { PcgDev st{}; return st; }
-
 template <class T>
 static void matvec(hipgp_plan* pl, int mode, const void* in, void* out, long B, cudaStream_t s) {
     if (!pl->have_spec) throw Error("plan has no spectrum: call hipgp_plan_set_first_row first");
     if (B < 0) throw Error("negative number of right-hand sides");
     if (B == 0) return;
     if (!in || !out) throw Error("null vector pointer");
-    RowsFusion ff, fi;
-    ff.mode = RF_PLAIN; ff.in = in; fi.mode = RI_PLAIN; fi.out = out;
     const bool wide = (mode == HIPGP_MV_RT || mode == HIPGP_MV_R);
     if (wide) ensure_wide<T>(pl, s);
     int n_in[3], n_out[3];
@@ -459,7 +413,7 @@ static void matvec(hipgp_plan* pl, int mode, const void* in, void* out, long B, 
         long_conv<T>(pl, long_geom<T>(pl, wide ? 1 : 0), (const T*)in, n_in[0], (T*)out, n_out[0], spec, kind, B, nullptr, s);
         return;
     }
-    run_pipeline<T>(pl, geom(pl, wide, Tag<T>()), n_in, n_out, spec, kind, B, ff, fi, null_state(), false, s);
+    run_pipeline<T>(pl, geom(pl, wide, Tag<T>()), n_in, n_out, spec, kind, B, plain_in(in), plain_out(out), null_state(), false, s);
 }
 
 template <class T>

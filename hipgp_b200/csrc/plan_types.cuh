@@ -216,12 +216,20 @@ struct Geom {
     LineFftHost<T> frow;
     DevBuf twL, twLp, part, pairq, pairs, pairw, quadq, quadw;
     int npair0 = 0, nquad = 0;
+    // Do the passes take the specialised kernel where their length has one?  fp32 pipelines keep the frequency workspace
+    // in lane layout (lane_fft.cuh), which the generic kernels do not read, so an fp32 geometry takes them only when every
+    // pass has one; fp64 lanes are plain interleaved complex numbers and the choice is made kernel by kernel (always true).
+    bool fast = false;
     bool built = false;
+    bool lane_layout() const { return sizeof(T) == 4 && fast; }
     void build(int D_, const int* L_, size_t* total) {
         D = D_;
         for (int d = 0; d < D; ++d) L[d] = L_[d];
         H = L[D - 1] / 2;
         P = ((long)H + 1 + 7) / 8 * 8;
+        bool all_listed = !fast_radices(H).empty();
+        for (int d = 0; d + 1 < D; ++d) all_listed = all_listed && !fast_radices(L[d]).empty();
+        fast = sizeof(T) == 8 || all_listed;
         for (int d = 0; d + 1 < D; ++d) fcol[d].build(L[d], total);
         frow.build(H, total);
         std::vector<cplx<T>> w(H);
@@ -301,7 +309,7 @@ struct LongGeom {
 };
 
 struct RowsFusion {
-    int mode = 0, dot_kind = 0, do_fft = 1;
+    int mode = 0, dot_kind = 0;
     const void* in = nullptr; void* out = nullptr; void* v0 = nullptr; void* v1 = nullptr; const void* v2 = nullptr;
 };
 
@@ -387,6 +395,6 @@ struct hipgp_plan {
 // instantiated by fast_inst.cu (compiled once per length group so that the build runs in parallel). ----
 namespace hipgp {
 template <class T, int LEN> void launch_rows_fast_len(hipgp_plan* pl, bool inverse, RowsParams<T>& P, cudaStream_t st);
-template <class T, int LEN> bool launch_cols_fast_len(hipgp_plan* pl, ColsParams<T>& P, long n_outer, long B, cudaStream_t st);   // false: lanes not 16-byte aligned
+template <class T, int LEN> void launch_cols_fast_len(hipgp_plan* pl, ColsParams<T>& P, long n_outer, long B, cudaStream_t st);   // throws: lanes not 16-byte aligned
 template <class T, int LEN> bool rows_fast_fits_len(long n_real);   // does the row pass of this length fit rows of n_real samples?
 }

@@ -134,7 +134,8 @@ def test_vec_kernels(lib):
     assert np.allclose(p, x + al * p0)
 
 
-@pytest.mark.parametrize("tag,dname", [("1d", "f64"), ("2d", "f64"), ("2d", "f32"), ("3d", "f64"), ("2d_odd", "f64")])
+@pytest.mark.parametrize("tag,dname", [("1d", "f64"), ("2d", "f64"), ("2d", "f32"), ("3d", "f64"), ("2d_odd", "f64"),
+                                      ("3d", "f32"), ("2d_odd", "f32"), ("1d", "f32")])
 def test_toeplitz_quadform(lib, tag, dname):
     """hipgp_toeplitz_quadform (forward passes, real spectrum product, one inverse, carry-pattern gather) against the
     reference's sym_toeplitz_derivative_quadratic_form on flattened 1-/2-/3-D grid vectors (golden, gpt_toeplitz.py:169-209)."""
