@@ -1,11 +1,16 @@
-// long1d_kernels.cuh -- four-step FFT convolution for 1-D embeddings too long for the one-block row pass.
+// long1d_kernels.cuh -- four-step FFT convolution along a last grid axis too long for the one-block row pass (1-D grids,
+// and the last axis of 2-D / 3-D grids).
 //
-// The embedding length factors as L = L1 * L2 and a sample index as n = L2 * n1 + n2 (n2 contiguous).  Data of one packed
-// pair of right-hand sides (x_a + i x_b) is a complex [L1][L2] array in the workspace, and a convolution is three passes:
+// The last axis' embedding length factors as L = L1 * L2 and a sample index as n = L2 * n1 + n2 (n2 contiguous).  Data of
+// one packed pair of right-hand sides (x_a + i x_b) along one row of the leading axes is a complex [L1][L2] array in the
+// workspace W[pair][row][L1][L2].  A pass runs on `nrows` rows per pair, CTA line index = pair * nrows + row (a 1-D grid
+// has one row).  Its input / output rows are the right-hand sides' [row][n] arrays, partner b one vector (nrows * n
+// values) after partner a.  A transform of the last axis is made of three passes:
 //   cols_fwd : strided L1-point DIF over n1 of the zero-padded input (only the first ceil(n_in / L2) rows are loaded), then
 //              the twiddle W_L^(n2 k1) on the way out.  Row p of the workspace holds k1 = rev1(p).
-//   rows     : contiguous L2-point DIF over n2, times the spectrum, L2-point DIT back (or the forward alone, at set-up).
-//              The spectrum is stored [p1][p2] in the same digit-reversed order, because set-up builds it with these passes.
+//   rows     : contiguous L2-point lines: DIF (LR_FWD), DIF times the spectrum then DIT back (LR_CONV, the middle of a 1-D
+//              convolution), or DIT alone (LR_INV, after the column passes of a 2-D / 3-D grid).  The spectrum is stored
+//              [p1][p2] in the same digit-reversed order, because set-up builds it with these passes.
 //   cols_inv : conjugate twiddle, strided L1-point DIT back to n1, crop to n_out, unpack into the two real output rows.
 // Every operator is a circular convolution with a real first column: K and C^-1 have real spectra, R^T a real or Hermitian
 // one and R its conjugate, so the real and imaginary parts of a packed pair never mix.
@@ -14,19 +19,24 @@
 
 namespace hipgp {
 
+enum LongRowsMode { LR_FWD = 0, LR_CONV = 1, LR_INV = 2 };
+
 template <class T>
 struct LongParams {
-    const T* in;              // cols_fwd: B real rows of n_in samples
-    T* out;                   // cols_inv: B real rows of n_out samples
-    cplx<T>* W;               // [pair][L1][L2]
+    const T* in;              // cols_fwd: B vectors of nrows real rows of n_in samples
+    T* out;                   // cols_inv: B vectors of nrows real rows of n_out samples
+    cplx<T>* W;               // [pair][W_rows][L1][L2]
     long B, n_in, n_out;
+    int nrows;                // rows per pair this pass runs on: grid.x = ntiles * pairs * nrows (< 2^31)
+    long W_rows;              // rows per pair in W (>= nrows)
     int L1, L2;
     LineFft<T> f1, f2;        // L1-point (strided) and L2-point (contiguous) line FFTs
     const cplx<T>* twh;       // W_L1^j, j < L1     (W_L^(n2 k1) = twh[j / L2] * twl[j % L2], j = n2 k1 < L)
     const cplx<T>* twl;       // W_L^j,  j < L2
     int TB, TBP;              // lines per CTA and padded line count (shared-memory line stride)
-    int ntiles;               // CTAs per pair: grid.x = ntiles * pairs
-    const void* spec; int spec_kind;   // rows: SPEC_NONE = forward only
+    int ntiles;               // CTAs per line
+    int rows_mode;            // rows: LongRowsMode
+    const void* spec; int spec_kind;   // rows, LR_CONV
     const int* done_flag;     // optional PCG early-exit flag
 };
 
@@ -42,22 +52,23 @@ __global__ void __launch_bounds__(256) long_cols_fwd_kernel(LongParams<T> P) {
     cplx<T>* s = reinterpret_cast<cplx<T>*>(smem_raw);
     const int tid = threadIdx.x, nthreads = blockDim.x;
     if (P.done_flag && *P.done_flag) return;
-    const long pair = blockIdx.x / P.ntiles;
+    const int line = blockIdx.x / P.ntiles, pair = line / P.nrows, row = line % P.nrows;
     const long c0 = (long)(blockIdx.x % P.ntiles) * P.TB;
     const int L1 = P.L1, TB = P.TB, TBP = P.TBP;
     const long rows_nz = (P.n_in + P.L2 - 1) / P.L2;
-    const T* ina = P.in + (size_t)(2 * pair) * P.n_in;
+    const long vec = (long)P.nrows * P.n_in;
+    const T* ina = P.in + (size_t)(2 * pair) * vec + (size_t)row * P.n_in;
     const bool has_b = 2 * pair + 1 < P.B;
     for (int w = tid; w < L1 * TB; w += nthreads) {
         const int c = w % TB, i = w / TB;
         const long n = (long)i * P.L2 + c0 + c;
         cplx<T> v = mk<T>(0, 0);
-        if (i < rows_nz && c0 + c < P.L2 && n < P.n_in) v = mk<T>(ina[n], has_b ? ina[P.n_in + n] : (T)0);
+        if (i < rows_nz && c0 + c < P.L2 && n < P.n_in) v = mk<T>(ina[n], has_b ? ina[vec + n] : (T)0);
         s[(size_t)i * TBP + c] = v;
     }
     __syncthreads();
     fft_forward(s, TBP, TB, P.f1, tid, nthreads);
-    cplx<T>* W = P.W + (size_t)pair * L1 * P.L2 + c0;
+    cplx<T>* W = P.W + ((size_t)pair * P.W_rows + row) * L1 * P.L2 + c0;
     for (int w = tid; w < L1 * TB; w += nthreads) {
         const int c = w % TB, p = w / TB;
         if (c0 + c < P.L2) W[(size_t)p * P.L2 + c] = s[(size_t)p * TBP + c] * long_twiddle(P, c0 + c, P.f1.rev[p]);
@@ -71,23 +82,23 @@ __global__ void __launch_bounds__(256) long_rows_kernel(LongParams<T> P) {
     const int tid = threadIdx.x, nthreads = blockDim.x;
     const int warp = tid >> 5, lane = tid & 31, nwarps = nthreads >> 5;
     if (P.done_flag && *P.done_flag) return;
-    const long pair = blockIdx.x / P.ntiles;
+    const int wline = blockIdx.x / P.ntiles, pair = wline / P.nrows, row = wline % P.nrows;
     const int r0 = (blockIdx.x % P.ntiles) * P.TB;
     const int L2 = P.L2, TB = P.TB, TBP = P.TBP;
     const int nl = P.L1 - r0 < TB ? P.L1 - r0 : TB;
-    cplx<T>* W = P.W + ((size_t)pair * P.L1 + r0) * L2;
+    cplx<T>* W = P.W + (((size_t)pair * P.W_rows + row) * P.L1 + r0) * L2;
     for (int line = warp; line < TB; line += nwarps)
         for (int q = lane; q < L2; q += 32) s[(size_t)q * TBP + line] = line < nl ? W[(size_t)line * L2 + q] : mk<T>(0, 0);
     __syncthreads();
-    fft_forward(s, TBP, TB, P.f2, tid, nthreads);
-    if (P.spec_kind != SPEC_NONE) {
+    if (P.rows_mode != LR_INV) fft_forward(s, TBP, TB, P.f2, tid, nthreads);
+    if (P.rows_mode == LR_CONV) {
         for (int w = tid; w < L2 * TB; w += nthreads) {
             const int line = w % TB, q = w / TB;
             if (line < nl) s[(size_t)q * TBP + line] = apply_spec(s[(size_t)q * TBP + line], P.spec, P.spec_kind, (size_t)(r0 + line) * L2 + q);
         }
         __syncthreads();
-        fft_inverse(s, TBP, TB, P.f2, tid, nthreads);
     }
+    if (P.rows_mode != LR_FWD) fft_inverse(s, TBP, TB, P.f2, tid, nthreads);
     for (int line = warp; line < nl; line += nwarps)
         for (int q = lane; q < L2; q += 32) W[(size_t)line * L2 + q] = s[(size_t)q * TBP + line];
 }
@@ -98,10 +109,10 @@ __global__ void __launch_bounds__(256) long_cols_inv_kernel(LongParams<T> P) {
     cplx<T>* s = reinterpret_cast<cplx<T>*>(smem_raw);
     const int tid = threadIdx.x, nthreads = blockDim.x;
     if (P.done_flag && *P.done_flag) return;
-    const long pair = blockIdx.x / P.ntiles;
+    const int line = blockIdx.x / P.ntiles, pair = line / P.nrows, row = line % P.nrows;
     const long c0 = (long)(blockIdx.x % P.ntiles) * P.TB;
     const int L1 = P.L1, TB = P.TB, TBP = P.TBP;
-    const cplx<T>* W = P.W + (size_t)pair * L1 * P.L2 + c0;
+    const cplx<T>* W = P.W + ((size_t)pair * P.W_rows + row) * L1 * P.L2 + c0;
     for (int w = tid; w < L1 * TB; w += nthreads) {
         const int c = w % TB, p = w / TB;
         cplx<T> v = mk<T>(0, 0);
@@ -111,7 +122,8 @@ __global__ void __launch_bounds__(256) long_cols_inv_kernel(LongParams<T> P) {
     __syncthreads();
     fft_inverse(s, TBP, TB, P.f1, tid, nthreads);
     const long rows_out = (P.n_out + P.L2 - 1) / P.L2;
-    T* outa = P.out + (size_t)(2 * pair) * P.n_out;
+    const long vec = (long)P.nrows * P.n_out;
+    T* outa = P.out + (size_t)(2 * pair) * vec + (size_t)row * P.n_out;
     const bool has_b = 2 * pair + 1 < P.B;
     for (int w = tid; w < (int)(rows_out < L1 ? rows_out : L1) * TB; w += nthreads) {
         const int c = w % TB, i = w / TB;
@@ -119,7 +131,7 @@ __global__ void __launch_bounds__(256) long_cols_inv_kernel(LongParams<T> P) {
         if (c0 + c < P.L2 && n < P.n_out) {
             const cplx<T> v = s[(size_t)i * TBP + c];
             outa[n] = v.x;
-            if (has_b) outa[P.n_out + n] = v.y;
+            if (has_b) outa[vec + n] = v.y;
         }
     }
 }

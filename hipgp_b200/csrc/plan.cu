@@ -43,14 +43,18 @@ static bool row_pass_fits(int H, long n_real) {
 template <class T>
 static bool row_embedding_fits(int L, long n_max) { return row_pass_fits<T>(L / 2, n_max) && row_pass_fits<double>(L / 2, L); }
 
-// the four-step path of long 1-D embeddings (long1d_api.inl)
+// the four-step path of long last axes (long1d_api.inl)
 template <class T> static LongGeom<T>& long_geom(hipgp_plan* pl, int which);
-template <class T> static void long_conv(hipgp_plan* pl, LongGeom<T>& g, const T* in, long n_in, T* out, long n_out, const void* spec,
-                                         int kind, long B, const int* done, cudaStream_t s);
-template <class T> static void long_build_spectrum(hipgp_plan* pl, bool wide, const double* col, DevBuf& dst, bool complex_spec, cudaStream_t s);
+template <class T> static void long_conv(hipgp_plan* pl, LongGeom<T>& g, Geom<T>& cg, const T* in, const int* n_in, T* out, const int* n_out,
+                                         const void* spec, int kind, long B, const int* done, cudaStream_t s);
 static void long_dct1(hipgp_plan* pl, const double* in, double* out, bool normalise, cudaStream_t s);
 template <class T> static void long_pcg_begin(hipgp_plan* pl, const PcgDev& st, long B, bool precond, cudaStream_t s);
 template <class T> static void long_pcg_iterate(hipgp_plan* pl, const PcgDev& st, int niter, cudaStream_t s);
+// what the entry points that need the row-pass layout (gradients, slab decomposition) say when they refuse such a plan
+static std::string four_step_plans(const hipgp_plan* pl) {
+    return pl->D == 1 ? "long 1-D plans (grids too long for the one-block row pass)"
+                      : "grids whose last axis is too long for the one-block row pass (four-step path)";
+}
 
 template <class T> static bool aligned2(const void* p) { return ((uintptr_t)p % (2 * sizeof(T))) == 0; }
 
@@ -279,23 +283,26 @@ static void dct_all_axes(hipgp_plan* pl, const double* in, double* out, double* 
 
 // the DCT-I of set_first_row / ensure_wide: Bluestein on long 1-D plans, the tiled kernels otherwise
 static void dct1(hipgp_plan* pl, const double* in, double* out, double* tmp, bool normalise, cudaStream_t s) {
-    if (pl->long_n) long_dct1(pl, in, out, normalise, s);
+    if (pl->D == 1 && pl->long_n) long_dct1(pl, in, out, normalise, s);
     else dct_all_axes(pl, in, out, tmp, normalise, s);
 }
 
+// The spectrum of a re-embedded first column, from the fp64 forward passes of the matvecs, in the layout they leave: half
+// spectra [L0]([L1])[P] on the row pass, full complex rows [L0]([L1])[L1 L2] in four-step order on the four-step path.
 template <class T>
 static void build_spectrum(hipgp_plan* pl, bool wide, const double* col, DevBuf& dst, bool complex_spec, cudaStream_t s) {
-    if (wide ? pl->long_w : pl->long_n) { long_build_spectrum<T>(pl, wide, col, dst, complex_spec, s); return; }
+    const bool four = wide ? pl->long_w : pl->long_n;
+    const int* Le = wide ? pl->Lw : pl->Ln;
     Geom<double>& g = wide ? pl->gw64 : pl->gn64;
     EmbedDims e{};
-    e.D = g.D;
+    e.D = pl->D;
     long total = 1;
     for (int d = 0; d < 3; ++d) { e.m[d] = 1; e.N[d] = 1; e.L[d] = 1; e.wide[d] = 0; }
     // right-align the D active axes into the 3 slots of EmbedDims
-    for (int d = 0; d < g.D; ++d) {
-        const int slot = 3 - g.D + d;
-        e.m[slot] = pl->m[d]; e.N[slot] = pl->N[d]; e.L[slot] = g.L[d]; e.wide[slot] = wide ? (pl->wide_real ? 2 : 1) : 0;
-        total *= g.L[d];
+    for (int d = 0; d < pl->D; ++d) {
+        const int slot = 3 - pl->D + d;
+        e.m[slot] = pl->m[d]; e.N[slot] = pl->N[d]; e.L[slot] = Le[d]; e.wide[slot] = wide ? (pl->wide_real ? 2 : 1) : 0;
+        total *= Le[d];
     }
     pl->tmpB.ensure(sizeof(double) * (size_t)total, &pl->dev_bytes);
     {
@@ -305,13 +312,21 @@ static void build_spectrum(hipgp_plan* pl, bool wide, const double* col, DevBuf&
         CK_LAUNCH(); pl->launches++;
     }
     // forward transform of the embedded column into W1 (raw spectrum, pipeline layout)
-    const long n = g.spec_elems();
-    pl->W1.ensure(sizeof(cplx<double>) * (size_t)n, &pl->dev_bytes);
+    long n;
+    double scale;
+    if (four) {
+        long_conv<double>(pl, long_geom<double>(pl, wide ? 1 : 0), g, pl->tmpB.as<double>(), Le, nullptr, nullptr, nullptr, SPEC_NONE, 1, nullptr, s);
+        n = total; scale = 1.0 / (double)total;
+    } else {
+        n = g.spec_elems();
+        pl->W1.ensure(sizeof(cplx<double>) * (size_t)n, &pl->dev_bytes);
+        cplx<double>* W1 = pl->W1.as<cplx<double>>();
+        run_rows<double>(pl, g, false, n / g.P, W1, n / g.P, 1, g.L[g.D - 1], plain_in(pl->tmpB.as<double>()), null_state(), s);
+        run_cols<double>(pl, g, CM_FWD, {W1, 0, g.L}, {W1, 0, g.L}, g.P, g.H + 1, 1, nullptr, SPEC_NONE, nullptr, s);
+        scale = 0.25;
+        for (int d = 0; d < g.D; ++d) scale /= (double)g.L[d];
+    }
     cplx<double>* W1 = pl->W1.as<cplx<double>>();
-    run_rows<double>(pl, g, false, n / g.P, W1, n / g.P, 1, g.L[g.D - 1], plain_in(pl->tmpB.as<double>()), null_state(), s);
-    run_cols<double>(pl, g, CM_FWD, {W1, 0, g.L}, {W1, 0, g.L}, g.P, g.H + 1, 1, nullptr, SPEC_NONE, nullptr, s);
-    double scale = 0.25;
-    for (int d = 0; d < g.D; ++d) scale /= (double)g.L[d];
     const unsigned nblk = (unsigned)((n + 255) / 256);
     if (complex_spec) {
         dst.ensure(sizeof(cplx<T>) * (size_t)n, &pl->dev_bytes);
@@ -323,15 +338,17 @@ static void build_spectrum(hipgp_plan* pl, bool wide, const double* col, DevBuf&
     CK_LAUNCH(); pl->launches++;
 }
 
+// (a four-step last axis builds its own geometry on first use; its geometry here holds the leading axes' column passes)
 template <class T>
 static void ensure_geoms(hipgp_plan* pl, bool wide) {
-    if (wide ? pl->long_w : pl->long_n) return;      // four-step geometry instead, built on first use
+    const bool four = wide ? pl->long_w : pl->long_n;
+    if (four && pl->D == 1) return;
     Geom<double>& g64 = wide ? pl->gw64 : pl->gn64;
     const int* L = wide ? pl->Lw : pl->Ln;
-    if (!g64.built) g64.build(pl->D, L, &pl->dev_bytes);
+    if (!g64.built) g64.build(pl->D, L, &pl->dev_bytes, !four);
     if (sizeof(T) == 4) {
         Geom<float>& g32 = wide ? pl->gw32 : pl->gn32;
-        if (!g32.built) g32.build(pl->D, L, &pl->dev_bytes);
+        if (!g32.built) g32.build(pl->D, L, &pl->dev_bytes, !four);
     }
 }
 
@@ -410,7 +427,7 @@ static void matvec(hipgp_plan* pl, int mode, const void* in, void* out, long B, 
         default: throw Error("unknown matvec mode");
     }
     if (wide ? pl->long_w : pl->long_n) {
-        long_conv<T>(pl, long_geom<T>(pl, wide ? 1 : 0), (const T*)in, n_in[0], (T*)out, n_out[0], spec, kind, B, nullptr, s);
+        long_conv<T>(pl, long_geom<T>(pl, wide ? 1 : 0), geom(pl, wide, Tag<T>()), (const T*)in, n_in, (T*)out, n_out, spec, kind, B, nullptr, s);
         return;
     }
     run_pipeline<T>(pl, geom(pl, wide, Tag<T>()), n_in, n_out, spec, kind, B, plain_in(in), plain_out(out), null_state(), false, s);
@@ -612,22 +629,24 @@ int hipgp_plan_create(int ndim, const int64_t* m, int dtype, int device, hipgp_p
             pl->Ln[d] = choose_length(2L * pl->m[d] - 1, row);
             pl->Lw[d] = choose_length((long)pl->N[d] + pl->m[d] - 1, row);
         }
-        // a 1-D embedding whose row pass would not fit shared memory takes the four-step path, at a length L1 * L2
-        if (D == 1) {
-            const long m0 = pl->m[0], N0 = pl->N[0];
+        // an embedding whose last-axis row pass would not fit shared memory takes the four-step path along that axis, at a
+        // length L1 * L2 (the other axes keep theirs)
+        {
+            const int a = D - 1;
+            const long ma = pl->m[a], Na = pl->N[a];
             auto fits = [&](int L, long n_max) { return dtype == HIPGP_F32 ? row_embedding_fits<float>(L, n_max) : row_embedding_fits<double>(L, n_max); };
             auto split = [&](long n, int which, int* L) {
                 int* f = pl->lsplit[which];
                 if (!long_split(n, &f[0], &f[1]))
-                    throw Error("1-D grid of " + std::to_string(m0) + " points is too long: the four-step path reaches " +
+                    throw Error((D == 1 ? "1-D grid of " : "last grid axis of ") + std::to_string(ma) + " points is too long: the four-step path reaches " +
                                 std::to_string((long)kLongMaxFactor * kLongMaxFactor) + "-point transforms (m <= " +
                                 std::to_string(((long)kLongMaxFactor * kLongMaxFactor + 5) / 4) + ")");
                 if (L) *L = f[0] * f[1];
             };
-            pl->long_n = !fits(pl->Ln[0], m0);
-            pl->long_w = pl->long_n || !fits(pl->Lw[0], N0);
-            if (pl->long_n) { split(2 * m0 - 1, 0, &pl->Ln[0]); split(2 * N0 - 1, 2, nullptr); }
-            if (pl->long_w) split(N0 + m0 - 1, 1, &pl->Lw[0]);
+            pl->long_n = !fits(pl->Ln[a], ma);
+            pl->long_w = pl->long_n || !fits(pl->Lw[a], Na);
+            if (pl->long_n) { split(2 * ma - 1, 0, &pl->Ln[a]); if (D == 1) split(2 * Na - 1, 2, nullptr); }
+            if (pl->long_w) split(Na + ma - 1, 1, &pl->Lw[a]);
         }
     } catch (...) { delete pl; throw; }
     *out = pl;

@@ -100,8 +100,8 @@ inline bool is_smooth(long n) {
 }
 
 // Shared-memory budgets of the row passes: the generic kernel (pick_rows_tiling, two padded rows at least) and the
-// specialised kernels (tile + side buffer).  A 1-D embedding whose row pass would exceed them takes the four-step path of
-// long1d_api.inl instead.  The test-only emulation build lowers HIPGP_ROW_SMEM_MAX with -D to run that path at small sizes.
+// specialised kernels (tile + side buffer).  An embedding whose last-axis row pass would exceed them takes the four-step
+// path of long1d_api.inl along that axis instead.  The test-only emulation build lowers HIPGP_ROW_SMEM_MAX with -D to run that path at small sizes.
 #ifndef HIPGP_ROW_SMEM_MAX
 #define HIPGP_ROW_SMEM_MAX (200 * 1024)
 #endif
@@ -222,15 +222,19 @@ struct Geom {
     bool fast = false;
     bool built = false;
     bool lane_layout() const { return sizeof(T) == 4 && fast; }
-    void build(int D_, const int* L_, size_t* total) {
+    // row_pass = false: a last axis on the four-step path (long1d_api.inl), which owns its own transforms; only the column
+    // passes of the leading axes are built.  They run on rows of interleaved complex numbers, so fp32 takes the generic
+    // column kernel throughout.
+    void build(int D_, const int* L_, size_t* total, bool row_pass = true) {
         D = D_;
         for (int d = 0; d < D; ++d) L[d] = L_[d];
         H = L[D - 1] / 2;
         P = ((long)H + 1 + 7) / 8 * 8;
         bool all_listed = !fast_radices(H).empty();
         for (int d = 0; d + 1 < D; ++d) all_listed = all_listed && !fast_radices(L[d]).empty();
-        fast = sizeof(T) == 8 || all_listed;
+        fast = sizeof(T) == 8 || (row_pass && all_listed);
         for (int d = 0; d + 1 < D; ++d) fcol[d].build(L[d], total);
+        if (!row_pass) { H = 0; P = L[D - 1]; built = true; return; }
         frow.build(H, total);
         std::vector<cplx<T>> w(H);
         for (int k = 0; k < H; ++k) {
@@ -287,7 +291,7 @@ struct Geom {
     void release(size_t* total) { for (auto& f : fcol) f.release(total); frow.release(total); twL.release(total); twLp.release(total); part.release(total); pairq.release(total); pairs.release(total); pairw.release(total); quadq.release(total); quadw.release(total); built = false; }
 };
 
-// four-step geometry of a long 1-D embedding (long1d_kernels.cuh): the two line FFTs and the twiddle tables, fp64-computed
+// four-step geometry of a long last axis (long1d_kernels.cuh): the two line FFTs and the twiddle tables, fp64-computed
 template <class T>
 struct LongGeom {
     int L1 = 0, L2 = 0;
@@ -335,8 +339,9 @@ struct hipgp_plan {
 
     Geom<float> gn32, gw32;    // narrow (K, Cinv) / wide (RT, R) geometries in the plan dtype
     Geom<double> gn64, gw64;   // fp64 geometries (set-up always runs in fp64; also the fp64 plan's own)
-    // 1-D embeddings too long for the row pass run the four-step path (long1d_api.inl): narrow / wide, each decided on its
-    // own; lsplit = (L1, L2) of the narrow, wide and Bluestein (DCT-I set-up, only when the narrow one is long) lengths
+    // embeddings whose last axis is too long for the row pass run that axis on the four-step path (long1d_api.inl): narrow /
+    // wide, each decided on its own; lsplit = (L1, L2) of the narrow, wide and Bluestein (DCT-I set-up of a 1-D plan, only
+    // when the narrow one is long) lengths.  gn / gw then hold the column passes of the leading axes only.
     bool long_n = false, long_w = false;
     int lsplit[3][2] = {{0, 0}, {0, 0}, {0, 0}};
     LongGeom<float> ln32, lw32;
